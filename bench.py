@@ -2,6 +2,7 @@
 """bench.py -- throughput of the QCTN contraction hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  Metric (BASELINE.json): samples/sec for the QCTN
 forward+backward contraction.  Workloads (SURVEY.md 8(d)):
@@ -26,6 +27,9 @@ e_{K-1}; Mx = TNTensor-normalised Hermite-function outer products).
 `--impl reference`: the reference's own CPU algorithm (oracle port of GreedyStrategy +
            torch.autograd, bit-identical to /root/reference on CPU, see oracle/) on the box's host
            cores, on a bounded sample of the same workload.
+`--dump-outputs DIR`: after the timed steps, what the last timed step returned (loss, per-sample values,
+           core gradients) as DIR/<name>.npy (see dump_outputs).  The inputs are seeded, so dumps of two
+           builds taken with the same arguments compare output for output.
 """
 from __future__ import annotations
 
@@ -81,6 +85,35 @@ def synth_inputs(graph, K, B, dtype):
     torch.manual_seed(42)
     x = torch.randn(B, nq)
     return names, table, nq, cores, x
+
+
+DUMP_BYTES = 60 << 20          # data of all dumped arrays together; with the .npy headers under 64 MB
+
+
+def dump_outputs(outdir, arrays):
+    """Write each named array (tensor or float) as outdir/<name>.npy: float64 data as float64, everything else as
+    float32, complex data with a trailing (real, imag) axis of 2.  When the arrays together exceed DUMP_BYTES, each
+    array larger than an equal share of it is replaced by that many of its elements (flattened, in index order),
+    chosen by a seeded permutation: the same elements on every run, so that dumps of two builds compare element for
+    element."""
+    import numpy as np
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    wide = (torch.float64, torch.complex128)
+    arrays = {k: torch.as_tensor(v).detach() for k, v in arrays.items()}
+    esz = {k: (2 if t.is_complex() else 1) * (8 if t.dtype in wide else 4) for k, t in arrays.items()}
+    sample = sum(t.numel() * esz[k] for k, t in arrays.items()) > DUMP_BYTES
+    share = DUMP_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        if sample and t.numel() * esz[name] > share:
+            gen = torch.Generator().manual_seed(0)
+            idx = torch.randperm(t.numel(), generator=gen)[:share // esz[name]].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        if t.is_complex():
+            t = torch.view_as_real(t.to(torch.complex128 if t.dtype in wide else torch.complex64))
+        else:
+            t = t.to(torch.float64 if t.dtype in wide else torch.float32)
+        np.save(os.path.join(outdir, name + ".npy"), t.cpu().numpy())
 
 
 class ClockSampler:
@@ -238,7 +271,11 @@ def main():
                          "the launch list of exactly one steady-state step)")
     ap.add_argument("--nccl-allreduce", action="store_true",
                     help="average gradients with NCCL instead of the one-shot NVLink kernel (tnq_allreduce_oneshot)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     wl = dict(WORKLOADS[args.workload])
     if args.batch:
         wl["batch"] = args.batch
@@ -403,9 +440,12 @@ def main():
         # the exchange is recorded into the training step's CUDA graph: a step is one graph launch
         fn.set_graph_epilogue(lambda loss0, grads: average(loss0, grads))
 
+    last = {}                                  # what the latest step_device() returned (--dump-outputs)
+
     def step_device():
         if train:
-            loss, grads, _vals, _sc = fn.loss_and_grads(cores_dict, states, mx_dev)
+            last["out"] = fn.loss_and_grads(cores_dict, states, mx_dev)
+            loss, grads, _vals, _sc = last["out"]
             if dist is not None:
                 if overlap["on"]:
                     average_overlapped(loss, grads)
@@ -414,8 +454,24 @@ def main():
             return loss
         with torch.no_grad():
             if wl["mode"] == "fwdx":
-                return engine.contract_from_x(qctn, states, x_dev, K=K)
-            return fn(cores_dict, states, mx_dev).tensor
+                last["out"] = engine.contract_from_x(qctn, states, x_dev, K=K)
+            else:
+                last["out"] = fn(cores_dict, states, mx_dev)
+            return last["out"]
+
+    def outputs_of(out):
+        """step_device()'s result as named arrays: loss, per-sample values, each core's gradient in qctn.cores
+        order (grad_000, ...: two core names can differ only in case), and the values' (scale, log_scale)."""
+        if not train:
+            if isinstance(out, torch.Tensor):
+                return {"values": out}
+            return {"values": out.tensor, "scale": torch.tensor([float(out.scale), float(out.log_scale)], dtype=torch.float64)}
+        loss, grads, vals, sc = out
+        arrays = {"loss": loss, "values": vals}
+        arrays.update((f"grad_{i:03d}", g) for i, g in enumerate(grads))
+        if sc is not None:
+            arrays["scale"] = torch.tensor([float(s) for s in sc], dtype=torch.float64)
+        return arrays
 
     if overlap["on"]:
         # once, on the ranks that are about to be timed: the overlapped per-core exchange must give what ONE packed NCCL
@@ -557,6 +613,9 @@ def main():
     ms_total, launches, clocks = timed(step_device, args.steps, args.warmup)
     ms_step = ms_total / args.steps
     value = B_global / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # now: the e2e steps below replay the same CUDA graph, whose output buffers they overwrite
+        dump_outputs(args.dump_outputs, outputs_of(last["out"]))
 
     e2e = None
     if not args.no_e2e:
@@ -564,8 +623,8 @@ def main():
             return step_e2e()
         # wall-clock inside CUDA events is not enough here (host work is part of e2e): use events
         # bracketing the whole call including the .item() read
-        ms_e2e, _, _ = timed(step_e2e_timed, max(3, args.steps // 2), 6)
-        ms_e2e_step = ms_e2e / max(3, args.steps // 2)
+        ms_e2e, _, _ = timed(step_e2e_timed, args.steps, 6)
+        ms_e2e_step = ms_e2e / args.steps
         e2e = {"value": B_global / (ms_e2e_step * 1e-3), "unit": "samples/s", "ms_per_step": ms_e2e_step,
                "h2d_bytes_per_step": h2d_bytes, "d2h_bytes_per_step": 4,
                "api": "EngineSiamese.contract_with_compiled_strategy" + ("_for_gradient" if train else ""),
@@ -685,8 +744,8 @@ def main():
             with torch.no_grad():
                 mats, _ = engine.generate_data(x_dev, K=K, ret_type="TNTensor")
                 return engine.contract_with_compiled_strategy(qctn, states, mats)
-        ms_unf, _, _ = timed(step_unfused, max(3, args.steps // 4), 3)
-        line["config"]["unfused_from_x_ms_per_step"] = ms_unf / max(3, args.steps // 4)
+        ms_unf, _, _ = timed(step_unfused, args.steps, 3)
+        line["config"]["unfused_from_x_ms_per_step"] = ms_unf / args.steps
     if e2e is not None:
         line["e2e"] = e2e
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
