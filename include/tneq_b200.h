@@ -186,6 +186,7 @@ int tnq_gemm_tf32x3_bk(const float* A, int a_mn, int64_t a_tiles, const float* B
  * (the generic route: a transposition of the 134 MB core plus a GEMM with two columns):
  *   tnq_fold_vec_f32 : out[a, c, ro]  = sum_{d, ri} P[a, d, c, ri] * Q[d, ri, ro]      P [A][D][C][2], Q [D][2][2]
  *   tnq_outer_acc_f32: T[a, d, c, ri] += sum_ro     P[a, c, ro]    * Q[d, ri, ro]      P [A][C][2],    T [A][D][C][2]
+ * D <= 4096 (Q is staged in shared memory); P, out and T 8-byte aligned.
  */
 int tnq_fold_vec_f32(const float* P, const float* Q, float* out, int64_t A, int64_t D, int64_t C, void* stream);
 int tnq_outer_acc_f32(const float* P, const float* Q, float* T, int64_t A, int64_t D, int64_t C, void* stream);

@@ -296,6 +296,15 @@ int fill_dims(Dims& d, int ndim, const int64_t* out_dims, const int64_t* in_stri
     return 0;
 }
 
+// Q of fold_vec / outer_acc sits in dynamic shared memory (16 D bytes): above the default 48 KB per block
+// (3072 < D <= 4096) a launch fails unless the kernel opts in to more
+template <typename Kernel>
+int allow_smem(Kernel kern, size_t bytes, const char* what) {
+    if (bytes <= 48 * 1024) return 0;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    return e == cudaSuccess ? 0 : tnq_internal_cuda_fail(e, what);
+}
+
 int grid_for(long long work, int per_block) {
     long long g = (work + per_block - 1) / per_block;
     const long long cap = 148LL * 16;
@@ -452,7 +461,9 @@ int tnq_cplx_fold_f32(const float* in, float* out, int ndim, const int64_t* out_
 int tnq_fold_vec_f32(const float* P, const float* Q, float* out, int64_t A, int64_t D, int64_t C, void* stream) {
     if (!P || !Q || !out || A <= 0 || D <= 0 || C <= 0 || D > 4096) return tnq_internal_fail("tnq_fold_vec_f32: bad arguments");
     if (((uintptr_t)P | (uintptr_t)out) & 7) return tnq_internal_fail("tnq_fold_vec_f32: pointers must be 8-byte aligned");
-    fold_vec_kernel<<<grid_for(A * C, 256), 256, sizeof(float) * 4 * (size_t)D, (cudaStream_t)stream>>>(P, Q, out, A, (int)D, C);
+    const size_t smem = sizeof(float) * 4 * (size_t)D;
+    if (int rc = allow_smem(fold_vec_kernel, smem, "cudaFuncSetAttribute(tnq_fold_vec_f32)")) return rc;
+    fold_vec_kernel<<<grid_for(A * C, 256), 256, smem, (cudaStream_t)stream>>>(P, Q, out, A, (int)D, C);
     tnq_internal_count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_fold_vec_f32 launch");
@@ -462,7 +473,9 @@ int tnq_fold_vec_f32(const float* P, const float* Q, float* out, int64_t A, int6
 int tnq_outer_acc_f32(const float* P, const float* Q, float* T, int64_t A, int64_t D, int64_t C, void* stream) {
     if (!P || !Q || !T || A <= 0 || D <= 0 || C <= 0 || D > 4096) return tnq_internal_fail("tnq_outer_acc_f32: bad arguments");
     if (((uintptr_t)P | (uintptr_t)T) & 7) return tnq_internal_fail("tnq_outer_acc_f32: pointers must be 8-byte aligned");
-    outer_acc_kernel<<<grid_for(A * C, 256), 256, sizeof(float) * 4 * (size_t)D, (cudaStream_t)stream>>>(P, Q, T, A, (int)D, C);
+    const size_t smem = sizeof(float) * 4 * (size_t)D;
+    if (int rc = allow_smem(outer_acc_kernel, smem, "cudaFuncSetAttribute(tnq_outer_acc_f32)")) return rc;
+    outer_acc_kernel<<<grid_for(A * C, 256), 256, smem, (cudaStream_t)stream>>>(P, Q, T, A, (int)D, C);
     tnq_internal_count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_outer_acc_f32 launch");

@@ -98,3 +98,124 @@ def upcast(x, td):
     if isinstance(x, oc.TNT):
         return oc.TNT(x.tensor.to(td), x.scale, x.log_scale)
     return x.to(td)
+
+
+def mps_f64(cores, states, mxs):
+    """The single-layer MPS sweep (einsum strings 'cdef,c,aeg,higj,h,d,i->ajf', 'cdef,aeg,higj,ahc,d,i->ajf',
+    'acd,adc->a') pairwise in the plan compiler's own order (3 K^4 per qubit and sample), on whatever device and
+    dtype the inputs have: in float64 / complex128 on the GPU, the yardstick of the large-bond route where the CPU
+    oracle's K^6 intermediates are out of reach.  Returns the amplitude (the engine reports |amp|^2 for complex
+    networks, amp for real ones).  Pinned to the oracle by tests/test_large_bond_yardstick.py."""
+    n = len(states)
+    a0, ac = cores[0], cores[0].conj()
+    v = torch.einsum("cdef,c,d->ef", a0, states[0], states[1])
+    w = torch.einsum("higj,h,i->gj", ac, states[0], states[1])
+    env = torch.einsum("ef,aeg,gj->ajf", v, mxs[0], w)
+    for qd in range(1, n - 1):
+        a = cores[qd]
+        v = torch.einsum("cdef,d->cef", a, states[qd + 1])
+        w = torch.einsum("higj,i->hgj", a.conj(), states[qd + 1])
+        t1 = torch.einsum("ahc,cef->ahef", env, v)
+        t2 = torch.einsum("ahef,aeg->ahgf", t1, mxs[qd])
+        env = torch.einsum("ahgf,hgj->ajf", t2, w)
+    return torch.einsum("acd,adc->a", env, mxs[n - 1])
+
+
+def mps_f64_value(amp):
+    """The value the engine reports for an amplitude: |amp|^2 for complex networks (reference quirk D10), amp for
+    real ones."""
+    return amp.real ** 2 + amp.imag ** 2 if amp.is_complex() else amp
+
+
+# ---- which GEMM variant a large-bond launch takes --------------------------------------------------------------------
+GEMM_TILE = 128          # BM = BN of csrc/tnq_gemm.cu
+GEMM_BK = 32             # BK of csrc/tnq_gemm.cu
+
+
+def gemm_splitk(M, N, K, batch=1, accumulate=False):
+    """Mirror of launch_tma's split-K rule (csrc/tnq_gemm.cu): a TMA-fed, non-small-K launch (K > 256) is split in
+    two along K when batch == 1, the tile is written (not accumulated), it covers at most 74 output tiles of
+    128 x 128 and K >= 32 k-blocks of 32."""
+    tiles = -(-M // GEMM_TILE) * -(-N // GEMM_TILE)
+    return batch == 1 and not accumulate and K > 256 and tiles <= 74 and K >= 32 * GEMM_BK
+
+
+def record_routes(monkeypatch, cls):
+    """Wrap the launch sites of a GemmPathRunner class (contractor/gemm_path.py) so that every kernel variant that
+    ran is counted.  Keys of the returned Counter:
+        ("view", split_k)              tnq_gemm_tf32x3_view (A permuted by the TMA unit)
+        ("bk", a_mn, b_mn, split_k)    tnq_gemm_tf32x3_bk (batch into K; x_mn: operand read MN-major in place)
+        ("gemm", split_k)              tnq_gemm_tf32x3 with batch 1 and K > 256 (the TMA-fed kernel)
+        ("fold_vec",) ("outer_acc",)   tnq_fold_vec_f32 / tnq_outer_acc_f32
+    Only launches that happened are counted (a refused view or bk falls back and is not)."""
+    from collections import Counter
+    from tneq_b200.contractor import gemm_path as gp
+    seen = Counter()
+    gemm, view, reduce_, fold, outer = cls._gemm, cls._gemm_view, cls._reduce_in_place, cls._fold_vec, cls._outer_acc
+
+    def _gemm(self, A, B, C, M, N, K, lda, ldb, ldc, batch=1, sA=0, sB=0, sC=0, accumulate=False):
+        gemm(self, A, B, C, M, N, K, lda, ldb, ldc, batch, sA, sB, sC, accumulate)
+        if batch == 1 and K > 256 and not (lda % 4 or ldb % 4):
+            seen[("gemm", gemm_splitk(M, N, K, batch, accumulate))] += 1
+
+    def _gemm_view(self, A, v, Bm, C, N, ldb, ldc):
+        ok = view(self, A, v, Bm, C, N, ldb, ldc)
+        if ok:
+            R1, R0, _, _, K1, K0, _ = v
+            seen[("view", gemm_splitk(R1 * R0, N, K1 * K0))] += 1
+        return ok
+
+    def _reduce_in_place(self, tp, Lp, pf, tq, Lq, qf, shared, NS):
+        out = reduce_(self, tp, Lp, pf, tq, Lq, qf, shared, NS)
+        if out is not None:
+            k = shared[0]
+            a_mn = self._mn_in_place(Lp, pf, k, NS) is not None
+            b_mn = self._mn_in_place(Lq, qf, k, NS) is not None
+            split = gemm_splitk(self._size(pf, NS), self._size(qf, NS), NS * self._extent(k, NS))
+            seen[("bk", int(a_mn), int(b_mn), split)] += 1
+        return out
+
+    def _fold_vec(self, n, val, lay):
+        out = fold(self, n, val, lay)
+        if out is not None:
+            seen[("fold_vec",)] += 1
+        return out
+
+    def _outer_acc(self, n, val, lay):
+        ok = outer(self, n, val, lay)
+        if ok:
+            seen[("outer_acc",)] += 1
+        return ok
+
+    for name, fn in (("_gemm", _gemm), ("_gemm_view", _gemm_view), ("_reduce_in_place", _reduce_in_place),
+                     ("_fold_vec", _fold_vec), ("_outer_acc", _outer_acc)):
+        monkeypatch.setattr(cls, name, fn)
+    assert gp.GemmPathRunner in cls.__mro__
+    return seen
+
+
+# The float64-parity cases of tests/test_gpu_large_bond.py, each with the kernel variants it exists to reach (keys of
+# record_routes) on the route that reads MN-major operands in place (gemm_path.MN_IN_PLACE) and on the transposing
+# route.  tests/test_gemm_path_plan.py checks the same expectations on meta tensors without a GPU.
+def _bk(split, pairs=((0, 1), (1, 0), (1, 1))):
+    return {("bk", a, b, split) for a, b in pairs}
+
+
+_FOLD = {("fold_vec",), ("outer_acc",)}
+LARGE_BOND_CASES = [
+    # dtype, chi, n, B, variants (MN in place), variants (transposing)
+    ("complex64", 64, 5, 256, _bk(True) | {("view", False), ("gemm", True)} | _FOLD,       # cfg4's per-qubit variants
+     {("view", False), ("gemm", True)} | _FOLD),
+    ("complex64", 64, 4, 5, _bk(False) | {("view", True)} | _FOLD,                        # smallest batch with bk
+     {("view", True)} | _FOLD),
+    ("complex64", 64, 6, 32, _bk(True) | {("view", True), ("gemm", True)} | _FOLD,
+     {("view", True), ("gemm", True)} | _FOLD),
+    ("complex64", 32, 5, 256, {("view", True), ("gemm", True)} | _FOLD,
+     {("view", True), ("gemm", True)} | _FOLD),
+    ("float32", 64, 5, 256, {("view", False), ("gemm", True)},
+     {("view", False), ("gemm", True)}),
+    ("float32", 128, 4, 8, _bk(False) | {("view", True), ("gemm", True)},
+     {("view", True), ("gemm", True), ("gemm", False)}),
+    ("complex64", 128, 3, 2, {("view", True)} | _FOLD,
+     {("view", True)} | _FOLD),
+]

@@ -9,17 +9,21 @@ import torch
 
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
 import gemm_path_dryrun as dr  # noqa: E402
+import pytest  # noqa: E402
 import tneq_b200  # noqa: E402
+from helpers import LARGE_BOND_CASES, record_routes  # noqa: E402
+from tneq_b200.contractor import gemm_path  # noqa: E402
 from tneq_b200.contractor.plan import ContractionPlan, signature_of  # noqa: E402
 
 
-def _walk(n, chi, B, fired=None):
+def _walk(n, chi, B, fired=None, dtype="complex64"):
     graph = tneq_b200.QCTNHelper.generate_example_graph(n=n, graph_type="mps", dim_char=str(chi))
     q = tneq_b200.QCTN(graph)
-    states = [torch.empty(chi, dtype=torch.complex64, device="meta") for _ in range(n)]
-    mxs = [torch.empty(B, chi, chi, dtype=torch.complex64, device="meta") for _ in range(n)]
+    td = getattr(torch, dtype)
+    states = [torch.empty(chi, dtype=td, device="meta") for _ in range(n)]
+    mxs = [torch.empty(B, chi, chi, dtype=td, device="meta") for _ in range(n)]
     sd, mi = signature_of(q.nqubits, states, mxs)
-    plan = ContractionPlan(q.adjacency_table, q.nqubits, {c: q.core_shape(c) for c in q.cores}, sd, mi, "complex64")
+    plan = ContractionPlan(q.adjacency_table, q.nqubits, {c: q.core_shape(c) for c in q.cores}, sd, mi, dtype)
     g = plan.graph("bwd")
     r = dr.DryRunner(g)
     inputs = {}
@@ -76,3 +80,18 @@ def test_grad_ready_hook_fires_once_per_core_in_reverse_use_order():
     names = sorted(g.grads, key=lambda k: str(k))
     assert order[names[-1]] < order[names[0]]
     assert fired[0][1] < len(r.log)
+
+
+@pytest.mark.parametrize("dtype,chi,n,B,want_mn,want_tr", LARGE_BOND_CASES,
+                         ids=[f"{c[0]}-chi{c[1]}-n{c[2]}-B{c[3]}" for c in LARGE_BOND_CASES])
+@pytest.mark.parametrize("mn_in_place", [True, False])
+def test_large_bond_case_plans_reach_their_variants(dtype, chi, n, B, want_mn, want_tr, mn_in_place, monkeypatch):
+    """The GEMM variants each float64-parity case of tests/test_gpu_large_bond.py exists to reach (the same recorder,
+    here around the dry runner): a routing change that drops a case's coverage fails here without a GPU."""
+    monkeypatch.setattr(gemm_path, "MN_IN_PLACE", mn_in_place)
+    seen = record_routes(monkeypatch, dr.DryRunner)
+    _walk(n, chi, B, dtype=dtype)
+    want = want_mn if mn_in_place else want_tr
+    assert want <= set(seen), sorted(want - set(seen))
+    if not mn_in_place:
+        assert not [k for k in seen if k[0] == "bk"]

@@ -9,7 +9,7 @@ import torch
 
 import tneq_b200
 from oracle import qctn_oracle as oc
-from helpers import well_conditioned_case, upcast, clone_mx, rel_err, NOISE_FACTOR
+from helpers import well_conditioned_case, upcast, clone_mx, rel_err, mps_f64, NOISE_FACTOR
 
 pytestmark = pytest.mark.gpu
 H = tneq_b200.QCTNHelper
@@ -127,25 +127,6 @@ def test_large_bond_identity_circuit(K, n, B, built_lib):
     assert rel_err(got.double().cpu(), want) < 2e-5      # |amplitude|^2: the amplitude's 1e-5 doubles
 
 
-def _mps_f64(cores, states, mxs):
-    """The single-layer MPS sweep (einsum strings 'cdef,c,aeg,higj,h,d,i->ajf', 'cdef,aeg,higj,ahc,d,i->ajf',
-    'acd,adc->a') in complex128 on the GPU, pairwise in the plan compiler's own order (3 K^4 per
-    qubit and sample): the yardstick where the CPU oracle's K^6 intermediates are out of reach."""
-    n = len(states)
-    a0, ac = cores[0], cores[0].conj()
-    v = torch.einsum("cdef,c,d->ef", a0, states[0], states[1])
-    w = torch.einsum("higj,h,i->gj", ac, states[0], states[1])
-    env = torch.einsum("ef,aeg,gj->ajf", v, mxs[0], w)
-    for qd in range(1, n - 1):
-        a = cores[qd]
-        v = torch.einsum("cdef,d->cef", a, states[qd + 1])
-        w = torch.einsum("higj,i->hgj", a.conj(), states[qd + 1])
-        t1 = torch.einsum("ahc,cef->ahef", env, v)
-        t2 = torch.einsum("ahef,aeg->ahgf", t1, mxs[qd])
-        env = torch.einsum("ahgf,hgj->ajf", t2, w)
-    return torch.einsum("acd,adc->a", env, mxs[n - 1])
-
-
 @pytest.mark.parametrize("K,n,B", [(32, 6, 6), (64, 5, 4)])
 def test_large_bond_loss_and_gradients_vs_float64(K, n, B, built_lib):
     """Values, loss and core gradients at bond 32 / 64 against a complex128 contraction of the same
@@ -169,7 +150,7 @@ def test_large_bond_loss_and_gradients_vs_float64(K, n, B, built_lib):
     fn = eng._compiled(q, st, mx, True, "symmetric")
     assert next(iter(fn.plans.values())).use_gemm_path
     c128 = [q.cores_weights[c].detach().to(torch.complex128).requires_grad_(True) for c in q.cores]
-    amp = _mps_f64(c128, [s.to(torch.complex128) for s in st], [m.to(torch.complex128) for m in mx])
+    amp = mps_f64(c128, [s.to(torch.complex128) for s in st], [m.to(torch.complex128) for m in mx])
     val = amp.real ** 2 + amp.imag ** 2
     assert rel_err(got.double().cpu(), val.detach().cpu()) < 2e-5
     want_loss = -(torch.log(torch.clamp(val, min=1e-10))).mean()
@@ -217,3 +198,102 @@ def test_permute_kernel_paths(built_lib):
                                    (c_int64 * 4)(*st), 2, 1, c_void_p(torch.cuda.current_stream().cuda_stream)))
     torch.cuda.synchronize()
     assert torch.equal(out, want)
+
+
+def _ptr(t):
+    from ctypes import c_void_p
+    return c_void_p(t.data_ptr())
+
+
+def _ptr_stream():
+    from ctypes import c_void_p
+    return c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+# The fold kernels sum 2 D float32 products in sequence: their rounding error relative to the largest output grows
+# like sqrt(D) (a float32 emulation of the kernel's order on the CPU gives 4.2e-7 at D = 64 and 2.7e-6 at D = 4096).
+def _fold_bound(D):
+    return 1e-6 * max(1.0, (D / 64) ** 0.5)
+
+
+@pytest.mark.parametrize("A,D,C", [(1, 1, 1), (3, 2, 5), (7, 3, 1), (5, 64, 129), (1, 128, 257), (3, 4096, 33), (2, 4096, 1)])
+def test_fold_vec_and_outer_acc_vs_float64(A, D, C, built_lib):
+    """tnq_fold_vec_f32 and tnq_outer_acc_f32 (include/tneq_b200.h) against float64 einsum: odd A and C, C = 1, D
+    from 1 to 4096 (above D = 3072 Q needs more than the default 48 KB of shared memory), outer_acc into a nonzero T."""
+    from tneq_b200 import _lib
+    lib = _lib.load()
+    torch.manual_seed(A * 1000 + D + C)
+    stream = _ptr_stream()
+    P = torch.randn(A, D, C, 2, device="cuda")
+    Q = torch.randn(D, 2, 2, device="cuda")
+    out = torch.full((A, C, 2), float("nan"), device="cuda")
+    launches = _lib.launch_count()
+    _lib.check(lib.tnq_fold_vec_f32(_ptr(P), _ptr(Q), _ptr(out), A, D, C, stream))
+    want = torch.einsum("adcr,dro->aco", P.double(), Q.double())
+    torch.cuda.synchronize()
+    assert _lib.launch_count() == launches + 1
+    assert rel_err(out.double(), want) < _fold_bound(D), rel_err(out.double(), want)
+    # the adjoint: T[a, d, c, ri] += sum_ro P[a, c, ro] Q[d, ri, ro], accumulated into a nonzero T
+    Pa = torch.randn(A, C, 2, device="cuda")
+    T0 = torch.randn(A, D, C, 2, device="cuda")
+    T = T0.clone()
+    _lib.check(lib.tnq_outer_acc_f32(_ptr(Pa), _ptr(Q), _ptr(T), A, D, C, stream))
+    want = T0.double() + torch.einsum("acO,drO->adcr", Pa.double(), Q.double())
+    torch.cuda.synchronize()
+    assert rel_err(T.double(), want) < 1e-6, rel_err(T.double(), want)
+
+
+def _expand_ref(z, ri, ro, conj):
+    """out[..., ri, ..., ro] = E[ri][ro] of z[...] (E = [[re, im], [-im, re]]), the two extent-2 dimensions inserted
+    at output positions ri < ro, in float64."""
+    z = z.conj() if conj else z
+    E = torch.stack([torch.stack([z.real, z.imag], -1), torch.stack([-z.imag, z.real], -1)], -2)   # [..., 2, 2]
+    nd = z.dim() + 2
+    order = [i for i in range(nd) if i not in (ri, ro)]          # output positions of z's dimensions
+    perm = [0] * nd
+    for src, dst in enumerate(order + [ri, ro]):
+        perm[dst] = src
+    return E.permute(*perm)
+
+
+@pytest.mark.parametrize("shape,ri,ro", [((3, 5), 2, 3), ((3, 5), 0, 2), ((4, 1, 7), 1, 4), ((33, 65), 0, 1), ((2, 3, 5), 1, 3)])
+@pytest.mark.parametrize("conj", [0, 1])
+def test_cplx_expand_and_fold_vs_float64(shape, ri, ro, conj, built_lib):
+    """tnq_cplx_expand_f32 (complex -> 2x2 real form fused with a permutation) and its adjoint tnq_cplx_fold_f32 against
+    float64: ri and ro at different output positions, a transposed (strided) input, conj, fold with accumulate."""
+    from tneq_b200 import _lib
+    lib = _lib.load()
+    from ctypes import c_int64
+    torch.manual_seed(sum(shape) * 10 + ri + ro + conj)
+    stream = _ptr_stream()
+    zt = torch.randn(*reversed(shape), dtype=torch.complex64, device="cuda")
+    z = zt.permute(*reversed(range(len(shape))))                  # z[...] read through strides
+    x = torch.view_as_real(zt)                                     # memory of z: (re, im) innermost
+    nd = len(shape) + 2
+    zdims = [i for i in range(nd) if i not in (ri, ro)]
+    dims = [0] * nd
+    st = [0] * nd
+    for k, pos in enumerate(zdims):
+        dims[pos], st[pos] = shape[k], x.stride(len(shape) - 1 - k)
+    dims[ri] = dims[ro] = 2
+    out = torch.empty(dims, device="cuda")
+    _lib.check(lib.tnq_cplx_expand_f32(_ptr(x), _ptr(out), nd, (c_int64 * nd)(*dims), (c_int64 * nd)(*st), ri, ro, conj,
+                                       stream))
+    want = _expand_ref(z.to(torch.complex128), ri, ro, conj)
+    torch.cuda.synchronize()
+    assert torch.equal(out.double(), want), (shape, ri, ro, conj)
+    # adjoint: dz[..., c] = sum_{ri ^ ro = c} sign * G[..., ri, ..., ro] in z's dimension order, added, then written
+    G = torch.randn(dims, device="cuda")
+    fdims = list(shape) + [2]
+    fst = [G.stride(pos) for pos in zdims] + [0]
+    g64 = G.double()
+    sel = lambda a, b: g64.select(ro, b).select(ri, a)             # ri < ro: select ro first
+    im = sel(0, 1) - sel(1, 0)
+    F = torch.stack([sel(0, 0) + sel(1, 1), -im if conj else im], -1)
+    prev = torch.randn(fdims, device="cuda")
+    got = prev.clone()
+    for acc, want in ((1, prev.double() + F), (0, F)):
+        _lib.check(lib.tnq_cplx_fold_f32(_ptr(G), _ptr(got), nd - 1, (c_int64 * (nd - 1))(*fdims),
+                                         (c_int64 * (nd - 1))(*fst), G.stride(ri), G.stride(ro), conj, acc, stream))
+        torch.cuda.synchronize()
+        assert rel_err(got.double(), want) < 1e-6, (acc, rel_err(got.double(), want))
