@@ -167,6 +167,16 @@ int tnq_mps_ladder(int K, int n, const float* const* cores_a, const float* const
 int tnq_gemm_tf32x3(const float* A, const float* B, float* C, int64_t M, int64_t N, int64_t K, int64_t lda,
                     int64_t ldb, int64_t ldc, int64_t batch, int64_t strideA, int64_t strideB, int64_t strideC,
                     int accumulate, void* stream);
+/*
+ * The same contraction in float64 (float64 / complex128 networks at large bond dimension) on the FP64 tensor
+ * cores (mma.sync m8n8k4 f64, csrc/tnq_gemm_f64.cu), same arguments with leading dimensions and batch strides
+ * in doubles.  Any M, N, K >= 1; 16-byte loads where K, lda / ldb, the batch strides (even) and the base
+ * addresses (16 bytes) allow, 8-byte loads otherwise; pointers 8-byte aligned.  Deterministic: a fixed
+ * summation order per output (a long k-loop on few tiles is split in two halves added with red.global.add.f64).
+ */
+int tnq_gemm_f64(const double* A, const double* B, double* C, int64_t M, int64_t N, int64_t K, int64_t lda,
+                 int64_t ldb, int64_t ldc, int64_t batch, int64_t strideA, int64_t strideB, int64_t strideC,
+                 int accumulate, void* stream);
 /* Launch resources of one variant of the GEMM kernel: out[4] = {registers per thread, max threads per block,
  * static shared bytes, threads per block the launch uses}. */
 /*
@@ -187,9 +197,12 @@ int tnq_gemm_tf32x3_bk(const float* A, int a_mn, int64_t a_tiles, const float* B
  *   tnq_fold_vec_f32 : out[a, c, ro]  = sum_{d, ri} P[a, d, c, ri] * Q[d, ri, ro]      P [A][D][C][2], Q [D][2][2]
  *   tnq_outer_acc_f32: T[a, d, c, ri] += sum_ro     P[a, c, ro]    * Q[d, ri, ro]      P [A][C][2],    T [A][D][C][2]
  * D <= 4096 (Q is staged in shared memory); P, out and T 8-byte aligned.
+ * The _f64 versions: the same on doubles (complex128), P, out and T 16-byte aligned.
  */
 int tnq_fold_vec_f32(const float* P, const float* Q, float* out, int64_t A, int64_t D, int64_t C, void* stream);
 int tnq_outer_acc_f32(const float* P, const float* Q, float* T, int64_t A, int64_t D, int64_t C, void* stream);
+int tnq_fold_vec_f64(const double* P, const double* Q, double* out, int64_t A, int64_t D, int64_t C, void* stream);
+int tnq_outer_acc_f64(const double* P, const double* Q, double* T, int64_t A, int64_t D, int64_t C, void* stream);
 int tnq_gemm_kernel_attrs(int aligned, int smallk, int* out);
 /*
  * The same GEMM with the index permutation of the A operand done by the TMA unit: A is a strided 4-level VIEW
@@ -209,8 +222,11 @@ int tnq_gemm_tf32x3_view(const float* A, int64_t R1, int64_t R0, int64_t sR1, in
  * `out` is compact row-major over out_dims[ndim]; in_strides[d] is the stride, in floats, of
  * output dimension d in `in`.  The innermost `vec` floats (1, 2 = one complex number, or 4)
  * move together and must be contiguous on both sides.  conj != 0 negates the imaginary parts.
+ * tnq_permute_f64: the same for float64 tensors, strides in doubles, vec 1 or 2 (2 = one complex128 number).
  */
 int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                    int vec, int conj, void* stream);
+int tnq_permute_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
                     int vec, int conj, void* stream);
 
 /*
@@ -219,10 +235,15 @@ int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_di
  * ri_dim / ro_dim are the positions of the two extra (extent-2) output dimensions; their
  * in_strides entries are ignored; `in`'s (re, im) pair is contiguous.  conj conjugates `in`.
  * tnq_cplx_fold_f32 is its adjoint (gradient path): out[..., c] (=|+=) sum over ri ^ ro == c.
+ * The _f64 versions: the same on doubles (complex128 in, float64 out), strides in doubles.
  */
 int tnq_cplx_expand_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
                         int ri_dim, int ro_dim, int conj, void* stream);
 int tnq_cplx_fold_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                      int64_t ri_stride, int64_t ro_stride, int conj, int accumulate, void* stream);
+int tnq_cplx_expand_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                        int ri_dim, int ro_dim, int conj, void* stream);
+int tnq_cplx_fold_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
                       int64_t ri_stride, int64_t ro_stride, int conj, int accumulate, void* stream);
 
 /*

@@ -14,7 +14,8 @@ LIB_PATH = os.path.join(_HERE, "libtneq_b200.so")
 
 EXPORTS = ["tnq_device_check", "tnq_plan_create", "tnq_plan_destroy", "tnq_plan_num_inputs",
            "tnq_plan_num_outputs", "tnq_plan_query", "tnq_plan_run", "tnq_gemm_tf32x3", "tnq_gemm_tf32x3_view", "tnq_gemm_tf32x3_bk", "tnq_gemm_kernel_attrs", "tnq_permute_f32", "tnq_fold_vec_f32", "tnq_outer_acc_f32", "tnq_cplx_expand_f32",
-           "tnq_cplx_fold_f32", "tnq_mps_chain", "tnq_mps_chain_workspace_bytes", "tnq_mps_chain_x", "tnq_mps_chain_sample", "tnq_mps_ladder",
+           "tnq_cplx_fold_f32", "tnq_gemm_f64", "tnq_permute_f64", "tnq_fold_vec_f64", "tnq_outer_acc_f64", "tnq_cplx_expand_f64",
+           "tnq_cplx_fold_f64", "tnq_mps_chain", "tnq_mps_chain_workspace_bytes", "tnq_mps_chain_x", "tnq_mps_chain_sample", "tnq_mps_ladder",
            "tnq_mps_ladder_workspace_bytes", "tnq_mps_ladder2", "tnq_mps_ladder2_workspace_bytes", "tnq_mps_ladder2_geometry", "tnq_allreduce_oneshot", "tnq_allreduce_oneshot_words", "tnq_allreduce_set_timeout_ms", "tnq_sgdg_step", "tnq_sgdg_step_flat", "tnq_launch_count",
            "tnq_last_error"]
 
@@ -59,6 +60,10 @@ def load():
                                         c_int, c_void_p]
     lib.tnq_cplx_fold_f32.argtypes = [c_void_p, c_void_p, c_int, POINTER(c_int64), POINTER(c_int64), c_int64, c_int64,
                                       c_int, c_int, c_void_p]
+    # float64 / complex128 siblings: same arguments, element strides in doubles
+    lib.tnq_gemm_f64.argtypes = lib.tnq_gemm_tf32x3.argtypes
+    for name in ("permute", "fold_vec", "outer_acc", "cplx_expand", "cplx_fold"):
+        getattr(lib, f"tnq_{name}_f64").argtypes = getattr(lib, f"tnq_{name}_f32").argtypes
     lib.tnq_mps_chain_workspace_bytes.argtypes = [c_int, c_int, c_int64]
     lib.tnq_mps_chain_workspace_bytes.restype = c_int64
     lib.tnq_mps_chain.argtypes = [c_int, c_int, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int64),

@@ -102,7 +102,7 @@ def _real_view(t: torch.Tensor) -> torch.Tensor:
 
 
 # Cores bigger than this (real elements) do not fit the shared-memory VM: the sweep is then
-# executed contraction by contraction on the tcgen05 GEMM path (gemm_path.py).
+# executed contraction by contraction on the tensor-core GEMM path (gemm_path.py), in the plan's dtype.
 VM_MAX_CORE_ELEMS = 4096
 
 
@@ -123,9 +123,8 @@ class _Bound:
         self.ladder, self._ladder_order, self._ladder_ws_bytes = None, None, {}
         if not (self.use_gemm_path or self.chain_rank or os.environ.get("TNQ_NO_CHAIN") == "1"):
             self.ladder = plan.mps_ladder()
-        if self.use_gemm_path and plan.real_dtype != "f32":
-            raise NotImplementedError("large-bond contraction runs on the tensor cores in float32 / complex64 only; "
-                                      f"got {plan.dtype} with a core of {biggest} elements")
+        # float32 / complex64 plans compute in float32, float64 / complex128 plans in float64
+        self.real_dtype = torch.float64 if plan.real_dtype == "f64" else torch.float32
 
     def scale_program(self):
         """[(tmp id produced, [(is_tmp, operand key)])] per greedy step, operands in einsum order."""
@@ -160,7 +159,7 @@ class _Bound:
     def gemm_runner(self, mode: str):
         from .gemm_path import GemmPathRunner
         if mode not in self._gemm:
-            self._gemm[mode] = GemmPathRunner(self.plan.graph(mode), self.device)
+            self._gemm[mode] = GemmPathRunner(self.plan.graph(mode), self.device, self.real_dtype)
         return self._gemm[mode]
 
     def program(self, mode: str) -> DeviceProgram:
@@ -348,7 +347,7 @@ class _Call:
         g = self.bound.gemm_runner("fwd").g
         for key, ids in g.inputs.items():
             if key[0] == "ones":
-                out[key] = self.bound.ones(g.size(g.nodes[ids[0]].idx), torch.float32)
+                out[key] = self.bound.ones(g.size(g.nodes[ids[0]].idx), self.bound.real_dtype)
         for q, m in self.mxs.items():
             m = m.detach()
             if m.shape[0] == 1 and self.B != 1:
@@ -395,7 +394,7 @@ class _Call:
         if self.bound.ladder:
             return self._ladder(cores, 2, seed=grad_out.reshape(-1).to(torch.float32).contiguous())[2]
         if self.bound.use_gemm_path:
-            seed = _real_view(grad_out.contiguous()).reshape(self.nsamples, -1).to(torch.float32).contiguous()
+            seed = _real_view(grad_out.contiguous()).reshape(self.nsamples, -1).to(self.bound.real_dtype).contiguous()
             return self._gemm_backward(cores, seed)[0]
         prog = self.bound.program("bwd")
         seed = _real_view(grad_out.contiguous()).reshape(self.nsamples, -1).to(prog.real_dtype).contiguous()
@@ -431,6 +430,7 @@ class _Call:
             inv = 1.0 / self.nsamples
 
             def seed_fn(res, layout):
+                # in the plan's real dtype (the forward result's): float64 plans seed the reverse sweep in float64
                 flat = res.reshape(self.nsamples, -1)
                 if flat.shape[1] == 2 and self.bound.plan.complex_mode:
                     val = flat[:, 0] * flat[:, 0] + flat[:, 1] * flat[:, 1]
@@ -771,7 +771,8 @@ class B200Strategy(ContractionStrategy):
                 graphs["seen"].clear()
 
         def set_grad_ready_hook(fn_or_none):
-            """fn(core name, flat float32 real view of that core's gradient), called DURING the reverse sweep of the
+            """fn(core name, flat real view of that core's gradient in the plan's real dtype -- float32, or float64 for
+            float64 / complex128 networks), called DURING the reverse sweep of the
             large-bond route as soon as the gradient of a core is final (reverse-use order): data-parallel training
             starts the core's all-reduce on a side stream there, so that the exchange of the GB-sized gradients runs
             under the rest of the sweep (bench.py --workload cfg4 --gpus N).  The fused small-bond kernels produce all

@@ -1,18 +1,23 @@
-"""Large-bond-dimension execution of a contraction graph: permute -> tcgen05 GEMM.
+"""Large-bond-dimension execution of a contraction graph: permute -> tensor-core GEMM.
 
 The shared-memory VM (vm_program.py / csrc/tnq_vm.cu) keeps every prepared core in shared
 memory, which stops working once cores have 64^4 elements.  In that regime every pairwise
 contraction of the sweep is a real GEMM, so the same contraction graph (cgraph.py) is executed
-node by node on global-memory tensors:
+node by node on global-memory tensors (here a float32 / complex64 plan):
 
     contract   ->  [tnq_permute_f32 to put the contracted indices innermost, only if needed]
                    tnq_gemm_tf32x3   (tcgen05, fp32-faithful 3xTF32, TMEM accumulators)
     lin        ->  tnq_permute_f32 (permute / conj), tnq_cplx_expand_f32, tnq_cplx_fold_f32
     reduce over the batch (core gradients) -> the batch is folded into the GEMM's K dimension
 
-float32 / complex64 only (tensor cores); complex contractions are real GEMMs of the operand
-against the 2x2-real expansion of the other (see cgraph.py).  PyTorch provides the buffers
-and the stream; all arithmetic on tensors is done by the kernels named above.
+float64 / complex128 plans run the same graph on the _f64 sibling of every kernel: tnq_gemm_f64 (FP64
+tensor cores, mma.sync f64), tnq_permute_f64, tnq_fold_vec_f64, tnq_outer_acc_f64, tnq_cplx_expand_f64 and
+tnq_cplx_fold_f64.  The two in-place GEMM variants (the TMA-permuted view, the MN-major core-gradient GEMM)
+are float32 only; in float64 their operands are transposed explicitly instead.
+
+Complex contractions are real GEMMs of the operand against the 2x2-real expansion of the other (see
+cgraph.py).  PyTorch provides the buffers and the stream; all arithmetic on tensors is done by the kernels
+named above.
 """
 from __future__ import annotations
 
@@ -31,35 +36,54 @@ MN_IN_PLACE = __import__("os").environ.get("TNQ_GEMM_MN", "1") == "1"
 
 
 class GemmPathRunner:
-    def __init__(self, graph: CGraph, device: torch.device):
+    dtype, f64, _sfx = torch.float32, False, "f32"
+
+    def __init__(self, graph: CGraph, device: torch.device, dtype: torch.dtype = torch.float32):
+        """dtype: the plan's real dtype, torch.float32 (float32 / complex64 plans) or torch.float64."""
         if device.type != "cuda":
             raise RuntimeError("the GEMM path runs on CUDA devices only (no CPU fallback)")
         self.g, self.device = graph, device
+        self._set_dtype(dtype)
         self.lib = _lib.load()
         with torch.cuda.device(device):
             _lib.check(self.lib.tnq_device_check())
         self.flops = 0.0
+
+    def _set_dtype(self, dtype: torch.dtype):
+        if dtype not in (torch.float32, torch.float64):
+            raise ValueError(f"the GEMM path computes in float32 or float64, not {dtype}")
+        self.dtype = dtype
+        self.f64 = dtype == torch.float64
+        self._sfx = "f64" if self.f64 else "f32"
+
+    def _entry(self, name: str):
+        """The library entry point tnq_<name>_f32 or tnq_<name>_f64 of this runner's dtype."""
+        return getattr(self.lib, f"tnq_{name}_{self._sfx}")
 
     # ---- raw kernel calls ------------------------------------------------------------
     def _stream(self):
         return c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def _permute(self, src: torch.Tensor, src_strides: Sequence[int], out_dims: Sequence[int], vec: int, conj: bool):
-        out = torch.empty(tuple(out_dims), dtype=torch.float32, device=self.device)
+        out = torch.empty(tuple(out_dims), dtype=self.dtype, device=self.device)
         n = len(out_dims)
-        _lib.check(self.lib.tnq_permute_f32(c_void_p(src.data_ptr()), c_void_p(out.data_ptr()), n,
-                                            (c_int64 * n)(*out_dims), (c_int64 * n)(*src_strides), vec, int(conj),
-                                            self._stream()))
+        _lib.check(self._entry("permute")(c_void_p(src.data_ptr()), c_void_p(out.data_ptr()), n,
+                                          (c_int64 * n)(*out_dims), (c_int64 * n)(*src_strides), vec, int(conj),
+                                          self._stream()))
         return out
 
     def _gemm(self, A, B, C, M, N, K, lda, ldb, ldc, batch=1, sA=0, sB=0, sC=0, accumulate=False):
-        _lib.check(self.lib.tnq_gemm_tf32x3(c_void_p(A.data_ptr()), c_void_p(B.data_ptr()), c_void_p(C.data_ptr()),
-                                            M, N, K, lda, ldb, ldc, batch, sA, sB, sC, int(accumulate), self._stream()))
+        gemm = self.lib.tnq_gemm_f64 if self.f64 else self.lib.tnq_gemm_tf32x3
+        _lib.check(gemm(c_void_p(A.data_ptr()), c_void_p(B.data_ptr()), c_void_p(C.data_ptr()),
+                        M, N, K, lda, ldb, ldc, batch, sA, sB, sC, int(accumulate), self._stream()))
         self.flops += 2.0 * M * N * K * batch
 
     def _gemm_view(self, A, view, Bm, C, N, ldb, ldc):
         """C = A_view x Bm^T with the permutation of A done by the TMA unit (tnq_gemm_tf32x3_view).  False: the
-        view is not expressible as a tensor map; nothing was launched."""
+        view is not expressible as a tensor map, or the runner computes in float64 (float32 only); nothing was
+        launched."""
+        if self.f64:
+            return False
         R1, R0, sR1, sR0, K1, K0, sK1 = view
         rc = self.lib.tnq_gemm_tf32x3_view(c_void_p(A.data_ptr()), R1, R0, sR1, sR0, K1, K0, sK1, c_void_p(Bm.data_ptr()),
                                            ldb, c_void_p(C.data_ptr()), ldc, N, self._stream())
@@ -101,9 +125,9 @@ class GemmPathRunner:
         j = L.index(d)
         A, D, C = self._size(L[:j], 1), g.dims[d], self._size(L[j + 1:-1], 1)
         out_layout = L[:j] + L[j + 1:-1] + [ro]
-        out = torch.empty([g.dims[i] for i in out_layout], dtype=torch.float32, device=self.device)
-        _lib.check(self.lib.tnq_fold_vec_f32(c_void_p(val[big.id].data_ptr()), c_void_p(val[small.id].data_ptr()),
-                                             c_void_p(out.data_ptr()), A, D, C, self._stream()))
+        out = torch.empty([g.dims[i] for i in out_layout], dtype=self.dtype, device=self.device)
+        _lib.check(self._entry("fold_vec")(c_void_p(val[big.id].data_ptr()), c_void_p(val[small.id].data_ptr()),
+                                           c_void_p(out.data_ptr()), A, D, C, self._stream()))
         self.flops += 2.0 * A * D * C * 4
         return out, out_layout
 
@@ -128,8 +152,8 @@ class GemmPathRunner:
         if not tgt.is_contiguous():
             return False
         A, D, C = self._size(T[:j], 1), g.dims[d], self._size(T[j + 1:-1], 1)
-        _lib.check(self.lib.tnq_outer_acc_f32(c_void_p(val[big.id].data_ptr()), c_void_p(val[small.id].data_ptr()),
-                                              c_void_p(tgt.data_ptr()), A, D, C, self._stream()))
+        _lib.check(self._entry("outer_acc")(c_void_p(val[big.id].data_ptr()), c_void_p(val[small.id].data_ptr()),
+                                            c_void_p(tgt.data_ptr()), A, D, C, self._stream()))
         self.flops += 2.0 * A * D * C * 4
         return True
 
@@ -147,8 +171,9 @@ class GemmPathRunner:
     def _reduce_in_place(self, tp, Lp, pf, tq, Lq, qf, shared, NS):
         """C[pf, qf] = sum over (batch, k) with at least one operand read in place, MN-major (the 537 MB intermediates of
         the bond-64 sweep are [batch][rows][k][128 rows]); the other operand is transposed explicitly when it is not of
-        that form (it is the small one).  None: not expressible, the caller transposes both."""
-        if len(shared) != 1 or not MN_IN_PLACE:
+        that form (it is the small one).  None: not expressible, or float64 (float32 only): the caller transposes
+        both."""
+        if len(shared) != 1 or not MN_IN_PLACE or self.f64:
             return None
         k = shared[0]
         a, b = self._mn_in_place(Lp, pf, k, NS), self._mn_in_place(Lq, qf, k, NS)
@@ -168,7 +193,7 @@ class GemmPathRunner:
         else:
             Bm, (b_tiles, rows_b) = tq, b
         M, N = self._size(pf, NS), self._size(qf, NS)
-        C = torch.empty((M, N), dtype=torch.float32, device=self.device)
+        C = torch.empty((M, N), dtype=self.dtype, device=self.device)
         rc = self.lib.tnq_gemm_tf32x3_bk(c_void_p(A.data_ptr()), int(a is not None), a_tiles, c_void_p(Bm.data_ptr()),
                                          int(b is not None), b_tiles, c_void_p(C.data_ptr()), M, N, NS, Kin, self._stream())
         if rc == -2:
@@ -250,7 +275,7 @@ class GemmPathRunner:
     # ---- node execution ----------------------------------------------------------------------
     def run(self, inputs: Dict[Tuple[str, object], torch.Tensor], B: int, nb: int, with_adjoint: bool,
             seed=None, on_grad_ready=None):
-        """inputs: real-view fp32 tensors per input key (batched ones with the sample dimension
+        """inputs: real-view tensors of the runner's dtype per input key (batched ones with the sample dimension
         first, nsamples = B * nb).  Returns (values dict, layouts dict).
         on_grad_ready(core key, flat real-view gradient): called as soon as a core's gradient is FINAL (all its
         contributions accumulated), in reverse-use order of the cores -- data-parallel training starts that core's
@@ -300,7 +325,7 @@ class GemmPathRunner:
             lay[n.id] = ([BATCH] if n.batched else []) + list(n.idx)
             return
         if n.is_accum:
-            val[n.id] = torch.zeros(tuple(g.dims[i] for i in n.idx) or (1,), dtype=torch.float32, device=self.device)
+            val[n.id] = torch.zeros(tuple(g.dims[i] for i in n.idx) or (1,), dtype=self.dtype, device=self.device)
             lay[n.id] = list(n.idx)
             return
         if n.kind == "seed":
@@ -354,11 +379,11 @@ class GemmPathRunner:
             target = lead + list(n.idx)
             dims = [self._extent(i, NS) for i in target]
             st = [0 if i in (ri, ro) else strides[i] for i in target]
-            out = torch.empty(tuple(dims), dtype=torch.float32, device=self.device)
+            out = torch.empty(tuple(dims), dtype=self.dtype, device=self.device)
             k = len(dims)
-            _lib.check(self.lib.tnq_cplx_expand_f32(c_void_p(t.data_ptr()), c_void_p(out.data_ptr()), k,
-                                                    (c_int64 * k)(*dims), (c_int64 * k)(*st), k - 2, k - 1, 0,
-                                                    self._stream()))
+            _lib.check(self._entry("cplx_expand")(c_void_p(t.data_ptr()), c_void_p(out.data_ptr()), k,
+                                                  (c_int64 * k)(*dims), (c_int64 * k)(*st), k - 2, k - 1, 0,
+                                                  self._stream()))
             return out, target
         if n.lin_kind == "fold":
             # source: gradient of the expanded tensor, layout contains ri, ro somewhere
@@ -366,11 +391,11 @@ class GemmPathRunner:
             target = lead + list(n.idx)
             dims = [self._extent(i, NS) for i in target]
             st = [strides[i] for i in target[:-1]] + [0]
-            out = torch.empty(tuple(dims), dtype=torch.float32, device=self.device)
+            out = torch.empty(tuple(dims), dtype=self.dtype, device=self.device)
             k = len(dims)
-            _lib.check(self.lib.tnq_cplx_fold_f32(c_void_p(t.data_ptr()), c_void_p(out.data_ptr()), k,
-                                                  (c_int64 * k)(*dims), (c_int64 * k)(*st), strides[ri], strides[ro],
-                                                  0, 0, self._stream()))
+            _lib.check(self._entry("cplx_fold")(c_void_p(t.data_ptr()), c_void_p(out.data_ptr()), k,
+                                                (c_int64 * k)(*dims), (c_int64 * k)(*st), strides[ri], strides[ro],
+                                                0, 0, self._stream()))
             return out, target
         raise NotImplementedError(f"lin kind {n.lin_kind!r} in the GEMM path")
 
@@ -391,7 +416,7 @@ class GemmPathRunner:
             A, rows_a = self._arrange(tp, Lp, pf, korder, NS)
             Bm, rows_b = self._arrange(tq, Lq, qf, korder, NS)
             M, N, K = self._size(pf, NS), self._size(qf, NS), self._size(korder, NS)
-            C = torch.empty((M, N), dtype=torch.float32, device=self.device)
+            C = torch.empty((M, N), dtype=self.dtype, device=self.device)
             self._gemm(A, Bm, C, M, N, K, K, K, N)
             out_layout = rows_a + rows_b
             return C.reshape([g.dims[i] for i in out_layout] or [1]), out_layout
@@ -400,7 +425,7 @@ class GemmPathRunner:
         lead = [BATCH] if p.batched else []
         korder = self._tail_order(Lp, shared)
         K = self._size(shared, NS)
-        if not q.batched:
+        if not q.batched and not self.f64:
             # the A operand read in place through a 4-D tensor map when its memory order is [rows][k][rows][k]
             sv = self._strided_view(Lp, lead + pf, korder, NS)
             if sv is not None:
@@ -410,7 +435,7 @@ class GemmPathRunner:
                 cur_b = [i for i in Lq if i in set(qf)]
                 Bm, rows_b = self._arrange(tq, Lq, want_b, korder, NS, exact=(want_b != cur_b))
                 M, N = self._size(rows_a, NS), self._size(rows_b, NS)
-                C = torch.empty((M, N), dtype=torch.float32, device=self.device)
+                C = torch.empty((M, N), dtype=self.dtype, device=self.device)
                 if self._gemm_view(tp, view, Bm, C, N, K, N):
                     out_layout = rows_a + rows_b
                     return C.reshape([self._extent(i, NS) for i in out_layout] or [1]), out_layout
@@ -420,7 +445,7 @@ class GemmPathRunner:
             Bm, rows_b = self._arrange(tq, Lq, [BATCH] + qf, korder, NS)
             assert rows_a[0] == BATCH and rows_b[0] == BATCH
             M, N = self._size(rows_a[1:], NS), self._size(rows_b[1:], NS)
-            C = torch.empty((NS, M, N), dtype=torch.float32, device=self.device)
+            C = torch.empty((NS, M, N), dtype=self.dtype, device=self.device)
             for b0 in range(0, NS, 32768):
                 nb_ = min(32768, NS - b0)
                 self._gemm(A[b0:] if b0 else A, Bm[b0:] if b0 else Bm, C[b0:] if b0 else C, M, N, K, K, K, N,
@@ -433,7 +458,7 @@ class GemmPathRunner:
             cur_b = [i for i in Lq if i in set(qf)]
             Bm, rows_b = self._arrange(tq, Lq, want_b, korder, NS, exact=(want_b != cur_b))
             M, N = self._size(rows_a, NS), self._size(rows_b, NS)
-            C = torch.empty((M, N), dtype=torch.float32, device=self.device)
+            C = torch.empty((M, N), dtype=self.dtype, device=self.device)
             self._gemm(A, Bm, C, M, N, K, K, K, N)
             out_layout = rows_a + rows_b
         return C.reshape([self._extent(i, NS) for i in out_layout] or [1]), out_layout

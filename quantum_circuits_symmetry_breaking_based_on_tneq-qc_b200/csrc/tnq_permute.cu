@@ -18,6 +18,9 @@
 //   tnq_cplx_expand_f32  Qx[..., ri, ..., ro] = E[ri][ro][c] * Q[..., c]  (E = 2x2 real form of a
 //                        complex number), permuted into GEMM operand layout in the same pass.
 //   tnq_cplx_fold_f32    the adjoint of the expansion (gradient path).
+// Every kernel is a template on the element type; the _f64 entry points are the same kernels on doubles
+// (float64 / complex128 networks): strides count doubles, vectors are at most two doubles (16 bytes), so a
+// complex128 number is vec = 2 and conj negates the second double of each 16-byte pair.
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -39,17 +42,28 @@ struct Dims {
     long long istride[MAXD];  // input stride (floats) of each output dimension
 };
 
-template <int VEC>
+template <typename T, int VEC>
 struct VecT;
 template <>
-struct VecT<1> { using type = float; };
+struct VecT<float, 1> { using type = float; };
 template <>
-struct VecT<2> { using type = float2; };
+struct VecT<float, 2> { using type = float2; };
 template <>
-struct VecT<4> { using type = float4; };
+struct VecT<float, 4> { using type = float4; };
+template <>
+struct VecT<double, 1> { using type = double; };
+template <>
+struct VecT<double, 2> { using type = double2; };
 
-template <int VEC>
-__device__ __forceinline__ typename VecT<VEC>::type conj_vec(typename VecT<VEC>::type v, int conj) {
+template <typename T>
+struct Pair;
+template <>
+struct Pair<float> { using type = float2; };
+template <>
+struct Pair<double> { using type = double2; };
+
+template <int VEC, typename V>
+__device__ __forceinline__ V conj_vec(V v, int conj) {
     if constexpr (VEC == 2) {
         if (conj) v.y = -v.y;
     } else if constexpr (VEC == 4) {
@@ -59,10 +73,10 @@ __device__ __forceinline__ typename VecT<VEC>::type conj_vec(typename VecT<VEC>:
 }
 
 // direct path: one thread per output vector; the innermost dimension is contiguous in the input
-template <int VEC>
-__global__ void __launch_bounds__(256) permute_direct_kernel(const float* __restrict__ in, float* __restrict__ out,
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256) permute_direct_kernel(const T* __restrict__ in, T* __restrict__ out,
                                                              Dims d, long long total, int conj) {
-    using V = typename VecT<VEC>::type;
+    using V = typename VecT<T, VEC>::type;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
          i += (long long)gridDim.x * blockDim.x) {
         long long rem = i, off = 0;
@@ -79,11 +93,11 @@ __global__ void __launch_bounds__(256) permute_direct_kernel(const float* __rest
 
 // tiled path: dimension `da` is the one that is contiguous in the INPUT, the last dimension is
 // contiguous in the OUTPUT; 32 x 32 vectors go through shared memory.
-template <int VEC>
-__global__ void __launch_bounds__(256) permute_tiled_kernel(const float* __restrict__ in, float* __restrict__ out,
+template <typename T, int VEC>
+__global__ void __launch_bounds__(256) permute_tiled_kernel(const T* __restrict__ in, T* __restrict__ out,
                                                             Dims d, int da, long long ostride_a, long long tiles_a,
                                                             long long tiles_b, long long ntiles, int conj) {
-    using V = typename VecT<VEC>::type;
+    using V = typename VecT<T, VEC>::type;
     __shared__ V tile[32][33];
     const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;   // 32 x 8
     const int db = d.nd - 1;
@@ -184,7 +198,8 @@ __global__ void __launch_bounds__(256) permute_tiled64_kernel(const float* __res
 
 // Qx[o] = sign * Q[i(o)] with the two extra output dimensions ri (dim pa) and ro (dim pb):
 // c = ri ^ ro, sign = -1 for (ri, ro) = (1, 0); conj flips the sign of c = 1.
-__global__ void __launch_bounds__(256) cplx_expand_kernel(const float* __restrict__ in, float* __restrict__ out, Dims d,
+template <typename T>
+__global__ void __launch_bounds__(256) cplx_expand_kernel(const T* __restrict__ in, T* __restrict__ out, Dims d,
                                                           long long total, int pa, int pb, int conj) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
          i += (long long)gridDim.x * blockDim.x) {
@@ -203,7 +218,7 @@ __global__ void __launch_bounds__(256) cplx_expand_kernel(const float* __restric
             rem = q;
         }
         const int c = ri ^ ro;
-        float v = __ldg(in + off + c);
+        T v = __ldg(in + off + c);
         if ((ri == 1 && ro == 0) != (conj && c == 1)) v = -v;
         out[i] = v;
     }
@@ -211,7 +226,8 @@ __global__ void __launch_bounds__(256) cplx_expand_kernel(const float* __restric
 
 // adjoint: dQ[..., c] = sum_{ri ^ ro = c} sign * dQx[..., ri, ..., ro]; `d` describes dQ (the last
 // dimension is c, extent 2) and istride the strides of dQx for the other dimensions.
-__global__ void __launch_bounds__(256) cplx_fold_kernel(const float* __restrict__ in, float* __restrict__ out, Dims d,
+template <typename T>
+__global__ void __launch_bounds__(256) cplx_fold_kernel(const T* __restrict__ in, T* __restrict__ out, Dims d,
                                                         long long total, long long sa, long long sb, int conj,
                                                         int accumulate) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -228,7 +244,7 @@ __global__ void __launch_bounds__(256) cplx_fold_kernel(const float* __restrict_
                 off += idx * d.istride[k];
             rem = q;
         }
-        float v;
+        T v;
         if (c == 0)
             v = __ldg(in + off) + __ldg(in + off + sa + sb);          // (0,0) + (1,1)
         else
@@ -244,42 +260,50 @@ __global__ void __launch_bounds__(256) cplx_fold_kernel(const float* __restrict_
 //     out[a, c, ro] = sum_{d, ri} P[a, d, c, ri] * Q[d, ri, ro]          P: [A][D][C][2] in place, Q: [D][2][2]
 // The generic route was transposition (2 x 134 MB at bond 64) + a GEMM with N = 2 (a 128-wide tensor-core tile for two
 // columns); here P is read ONCE, coalesced along c, Q sits in shared memory.
-__global__ void __launch_bounds__(256) fold_vec_kernel(const float* __restrict__ P, const float* __restrict__ Q,
-                                                      float* __restrict__ out, long long A, int D, long long C) {
-    extern __shared__ float q[];                     // [D][4]
+template <typename T>
+__global__ void __launch_bounds__(256) fold_vec_kernel(const T* __restrict__ P, const T* __restrict__ Q,
+                                                      T* __restrict__ out, long long A, int D, long long C) {
+    using T2 = typename Pair<T>::type;
+    extern __shared__ __align__(16) unsigned char q_raw[];
+    T* q = reinterpret_cast<T*>(q_raw);              // [D][4]
     for (int i = threadIdx.x; i < D * 4; i += blockDim.x) q[i] = __ldg(Q + i);
     __syncthreads();
     const long long total = A * C;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long a = i / C, c = i - a * C;
-        const float2* src = reinterpret_cast<const float2*>(P) + a * D * C + c;
-        float o0 = 0.f, o1 = 0.f;
+        const T2* src = reinterpret_cast<const T2*>(P) + a * D * C + c;
+        T o0 = 0, o1 = 0;
 #pragma unroll 8
         for (int d = 0; d < D; ++d) {
-            const float2 v = __ldg(src + (long long)d * C);
-            o0 = fmaf(v.x, q[4 * d], fmaf(v.y, q[4 * d + 2], o0));
-            o1 = fmaf(v.x, q[4 * d + 1], fmaf(v.y, q[4 * d + 3], o1));
+            const T2 v = __ldg(src + (long long)d * C);
+            o0 = fma(v.x, q[4 * d], fma(v.y, q[4 * d + 2], o0));
+            o1 = fma(v.x, q[4 * d + 1], fma(v.y, q[4 * d + 3], o1));
         }
-        reinterpret_cast<float2*>(out)[i] = make_float2(o0, o1);
+        T2 o;
+        o.x = o0, o.y = o1;
+        reinterpret_cast<T2*>(out)[i] = o;
     }
 }
 
 // the adjoint (an outer product accumulated in place): T[a, d, c, ri] += sum_ro P[a, c, ro] * Q[d, ri, ro]
-__global__ void __launch_bounds__(256) outer_acc_kernel(const float* __restrict__ P, const float* __restrict__ Q,
-                                                       float* __restrict__ T, long long A, int D, long long C) {
-    extern __shared__ float q[];                     // [D][4]
+template <typename E>
+__global__ void __launch_bounds__(256) outer_acc_kernel(const E* __restrict__ P, const E* __restrict__ Q,
+                                                       E* __restrict__ T, long long A, int D, long long C) {
+    using E2 = typename Pair<E>::type;
+    extern __shared__ __align__(16) unsigned char q_raw[];
+    E* q = reinterpret_cast<E*>(q_raw);              // [D][4]
     for (int i = threadIdx.x; i < D * 4; i += blockDim.x) q[i] = __ldg(Q + i);
     __syncthreads();
     const long long total = A * C;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long a = i / C, c = i - a * C;
-        const float2 p = __ldg(reinterpret_cast<const float2*>(P) + i);
-        float2* dst = reinterpret_cast<float2*>(T) + a * D * C + c;
+        const E2 p = __ldg(reinterpret_cast<const E2*>(P) + i);
+        E2* dst = reinterpret_cast<E2*>(T) + a * D * C + c;
 #pragma unroll 8
         for (int d = 0; d < D; ++d) {
-            float2 t = dst[(long long)d * C];
-            t.x = fmaf(p.x, q[4 * d], fmaf(p.y, q[4 * d + 1], t.x));
-            t.y = fmaf(p.x, q[4 * d + 2], fmaf(p.y, q[4 * d + 3], t.y));
+            E2 t = dst[(long long)d * C];
+            t.x = fma(p.x, q[4 * d], fma(p.y, q[4 * d + 1], t.x));
+            t.y = fma(p.x, q[4 * d + 2], fma(p.y, q[4 * d + 3], t.y));
             dst[(long long)d * C] = t;
         }
     }
@@ -296,13 +320,13 @@ int fill_dims(Dims& d, int ndim, const int64_t* out_dims, const int64_t* in_stri
     return 0;
 }
 
-// Q of fold_vec / outer_acc sits in dynamic shared memory (16 D bytes): above the default 48 KB per block
-// (3072 < D <= 4096) a launch fails unless the kernel opts in to more
+// Q of fold_vec / outer_acc sits in dynamic shared memory (16 D bytes in float32, 32 D in float64): above the default
+// 48 KB per block (float32: 3072 < D <= 4096, float64: 1536 < D <= 4096) a launch fails unless the kernel opts in to more
 template <typename Kernel>
-int allow_smem(Kernel kern, size_t bytes, const char* what) {
+int allow_smem(Kernel kern, size_t bytes, const std::string& what) {
     if (bytes <= 48 * 1024) return 0;
     const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    return e == cudaSuccess ? 0 : tnq_internal_cuda_fail(e, what);
+    return e == cudaSuccess ? 0 : tnq_internal_cuda_fail(e, what.c_str());
 }
 
 int grid_for(long long work, int per_block) {
@@ -311,27 +335,29 @@ int grid_for(long long work, int per_block) {
     return (int)(g < 1 ? 1 : (g > cap ? cap : g));
 }
 
-}  // namespace
 
-extern "C" {
-
-int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
-                    int vec, int conj, void* stream) {
-    if (!in || !out || !out_dims || !in_strides) return tnq_internal_fail("tnq_permute_f32: bad arguments");
-    if (vec != 1 && vec != 2 && vec != 4) return tnq_internal_fail("tnq_permute_f32: vec must be 1, 2 or 4");
-    if (conj && vec == 1) return tnq_internal_fail("tnq_permute_f32: conj needs vec >= 2 (interleaved complex)");
+template <typename T>
+int permute_impl(const T* in, T* out, int ndim, const int64_t* out_dims, const int64_t* in_strides, int vec, int conj,
+                 void* stream, const char* name) {
+    const std::string nm(name);
+    constexpr int ES = (int)sizeof(T);
+    constexpr int VMAX = 16 / ES;                    // widest vector: 16 bytes
+    if (!in || !out || !out_dims || !in_strides) return tnq_internal_fail(nm + ": bad arguments");
+    if (vec != 1 && vec != 2 && vec != 4) return tnq_internal_fail(nm + ": vec must be 1, 2 or 4");
+    if (vec > VMAX) return tnq_internal_fail(nm + ": vec must be 1 or 2");
+    if (conj && vec == 1) return tnq_internal_fail(nm + ": conj needs vec >= 2 (interleaved complex)");
     Dims d;
     if (int rc = fill_dims(d, ndim, out_dims, in_strides)) return rc;
-    if (((uintptr_t)in | (uintptr_t)out) & (uintptr_t)(vec * 4 - 1))
-        return tnq_internal_fail("tnq_permute_f32: pointers must be aligned to the vector width");
+    if (((uintptr_t)in | (uintptr_t)out) & (uintptr_t)(vec * ES - 1))
+        return tnq_internal_fail(nm + ": pointers must be aligned to the vector width");
     long long total = 1;
     for (int k = 0; k < ndim; ++k) {
-        if (k < ndim - 1 && vec > 1 && (d.istride[k] % vec)) return tnq_internal_fail("tnq_permute_f32: stride not a multiple of vec");
+        if (k < ndim - 1 && vec > 1 && (d.istride[k] % vec)) return tnq_internal_fail(nm + ": stride not a multiple of vec");
         total *= d.size[k];
     }
     if (vec > 1 && (d.size[ndim - 1] % vec || d.istride[ndim - 1] != 1))
-        return tnq_internal_fail("tnq_permute_f32: the last dimension must be contiguous and a multiple of vec");
-    // ---- canonical form (all in floats): drop extent-1 dimensions, merge neighbours that are adjacent in the input
+        return tnq_internal_fail(nm + ": the last dimension must be contiguous and a multiple of vec");
+    // ---- canonical form (all in elements): drop extent-1 dimensions, merge neighbours that are adjacent in the input
     // in the same order as in the output (stride[k] == stride[k+1] * size[k+1]): a (.., 64, 2) pair of (index, re/im)
     // becomes one run of 128 contiguous floats, so that a true transposition finds a long input-contiguous dimension
     // for its shared-memory tiles instead of falling back to strided scalar loads (measured on the 537 MB
@@ -357,8 +383,8 @@ int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_di
     // ---- widest vector that keeps the meaning: the last dimension contiguous in the input, its extent and every
     // other stride a multiple of the width, both pointers aligned (a requested vec = 2 with conj stays >= 2)
     if (d.istride[d.nd - 1] == 1) {
-        for (int w = 4; w > vec; w >>= 1) {
-            bool ok = d.size[d.nd - 1] % w == 0 && !(((uintptr_t)in | (uintptr_t)out) & (uintptr_t)(w * 4 - 1));
+        for (int w = VMAX; w > vec; w >>= 1) {
+            bool ok = d.size[d.nd - 1] % w == 0 && !(((uintptr_t)in | (uintptr_t)out) & (uintptr_t)(w * ES - 1));
             for (int k = 0; k < d.nd - 1 && ok; ++k) ok = d.istride[k] % w == 0;
             if (ok) {
                 vec = w;
@@ -366,7 +392,7 @@ int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_di
             }
         }
     }
-    // fold the innermost `vec` floats into one element
+    // fold the innermost `vec` elements into one vector
     if (vec > 1) {
         d.size[d.nd - 1] /= vec;
         d.istride[d.nd - 1] = vec;
@@ -382,104 +408,157 @@ int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_di
                         d.size[da] < 8;
     if (direct) {
         const int grid = grid_for(total, 256 * 4);
-        if (vec == 1) permute_direct_kernel<1><<<grid, 256, 0, st>>>(in, out, d, total, conj);
-        if (vec == 2) permute_direct_kernel<2><<<grid, 256, 0, st>>>(in, out, d, total, conj);
-        if (vec == 4) permute_direct_kernel<4><<<grid, 256, 0, st>>>(in, out, d, total, conj);
+        if (vec == 1) permute_direct_kernel<T, 1><<<grid, 256, 0, st>>>(in, out, d, total, conj);
+        if (vec == 2) permute_direct_kernel<T, 2><<<grid, 256, 0, st>>>(in, out, d, total, conj);
+        if constexpr (VMAX == 4)
+            if (vec == 4) permute_direct_kernel<T, 4><<<grid, 256, 0, st>>>(in, out, d, total, conj);
     } else {
         long long ostride_a = 1;
         for (int k = d.nd - 1; k > da; --k) ostride_a *= d.size[k];
-        bool wide = vec == 1 && !conj && d.size[da] % 4 == 0 && d.size[d.nd - 1] % 4 == 0 && ostride_a % 4 == 0 &&
-                    d.size[da] >= 32 && d.size[d.nd - 1] >= 32 && !(((uintptr_t)in | (uintptr_t)out) & 15);
-        for (int k = 0; k < d.nd && wide; ++k)
-            if (k != da) wide = d.istride[k] % 4 == 0;
-        if (wide) {
-            long long os = 1;                        // every output stride above the last dimension is a multiple of four
-            for (int k = d.nd - 1; k >= 1 && wide; --k) {
-                os *= d.size[k];
-                wide = os % 4 == 0;
+        if constexpr (sizeof(T) == 4) {
+            bool wide = vec == 1 && !conj && d.size[da] % 4 == 0 && d.size[d.nd - 1] % 4 == 0 && ostride_a % 4 == 0 &&
+                        d.size[da] >= 32 && d.size[d.nd - 1] >= 32 && !(((uintptr_t)in | (uintptr_t)out) & 15);
+            for (int k = 0; k < d.nd && wide; ++k)
+                if (k != da) wide = d.istride[k] % 4 == 0;
+            if (wide) {
+                long long os = 1;                    // every output stride above the last dimension is a multiple of four
+                for (int k = d.nd - 1; k >= 1 && wide; --k) {
+                    os *= d.size[k];
+                    wide = os % 4 == 0;
+                }
             }
-        }
-        if (wide) {
-            const long long tiles_a = (d.size[da] + 63) / 64, tiles_b = (d.size[d.nd - 1] + 63) / 64;
-            long long ntiles = tiles_a * tiles_b;
-            for (int k = 0; k < d.nd - 1; ++k)
-                if (k != da) ntiles *= d.size[k];
-            permute_tiled64_kernel<<<grid_for(ntiles, 1), 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles);
-            tnq_internal_count_launch();
-            cudaError_t e64 = cudaGetLastError();
-            if (e64 != cudaSuccess) return tnq_internal_cuda_fail(e64, "tnq_permute_f32 launch");
-            return 0;
+            if (wide) {
+                const long long tiles_a = (d.size[da] + 63) / 64, tiles_b = (d.size[d.nd - 1] + 63) / 64;
+                long long ntiles = tiles_a * tiles_b;
+                for (int k = 0; k < d.nd - 1; ++k)
+                    if (k != da) ntiles *= d.size[k];
+                permute_tiled64_kernel<<<grid_for(ntiles, 1), 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles);
+                tnq_internal_count_launch();
+                cudaError_t e64 = cudaGetLastError();
+                if (e64 != cudaSuccess) return tnq_internal_cuda_fail(e64, (nm + " launch").c_str());
+                return 0;
+            }
         }
         const long long tiles_a = (d.size[da] + 31) / 32, tiles_b = (d.size[d.nd - 1] + 31) / 32;
         long long ntiles = tiles_a * tiles_b;
         for (int k = 0; k < d.nd - 1; ++k)
             if (k != da) ntiles *= d.size[k];
         const int grid = grid_for(ntiles, 1);
-        if (vec == 1) permute_tiled_kernel<1><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
-        if (vec == 2) permute_tiled_kernel<2><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
-        if (vec == 4) permute_tiled_kernel<4><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
+        if (vec == 1) permute_tiled_kernel<T, 1><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
+        if (vec == 2) permute_tiled_kernel<T, 2><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
+        if constexpr (VMAX == 4)
+            if (vec == 4) permute_tiled_kernel<T, 4><<<grid, 256, 0, st>>>(in, out, d, da, ostride_a, tiles_a, tiles_b, ntiles, conj);
     }
     tnq_internal_count_launch();
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_permute_f32 launch");
+    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, (nm + " launch").c_str());
     return 0;
 }
 
-int tnq_cplx_expand_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
-                        int ri_dim, int ro_dim, int conj, void* stream) {
-    if (!in || !out) return tnq_internal_fail("tnq_cplx_expand_f32: bad arguments");
+template <typename T>
+int cplx_expand_impl(const T* in, T* out, int ndim, const int64_t* out_dims, const int64_t* in_strides, int ri_dim,
+                     int ro_dim, int conj, void* stream, const char* name) {
+    const std::string nm(name);
+    if (!in || !out) return tnq_internal_fail(nm + ": bad arguments");
     Dims d;
     if (int rc = fill_dims(d, ndim, out_dims, in_strides)) return rc;
     if (ri_dim < 0 || ro_dim < 0 || ri_dim >= ndim || ro_dim >= ndim || ri_dim == ro_dim || d.size[ri_dim] != 2 ||
         d.size[ro_dim] != 2)
-        return tnq_internal_fail("tnq_cplx_expand_f32: ri/ro must be two distinct output dimensions of extent 2");
+        return tnq_internal_fail(nm + ": ri/ro must be two distinct output dimensions of extent 2");
     long long total = 1;
     for (int k = 0; k < ndim; ++k) total *= d.size[k];
-    cplx_expand_kernel<<<grid_for(total, 256 * 4), 256, 0, (cudaStream_t)stream>>>(in, out, d, total, ri_dim, ro_dim, conj);
+    cplx_expand_kernel<T><<<grid_for(total, 256 * 4), 256, 0, (cudaStream_t)stream>>>(in, out, d, total, ri_dim, ro_dim, conj);
     tnq_internal_count_launch();
     cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_cplx_expand_f32 launch");
+    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, (nm + " launch").c_str());
     return 0;
+}
+
+template <typename T>
+int cplx_fold_impl(const T* in, T* out, int ndim, const int64_t* out_dims, const int64_t* in_strides, int64_t ri_stride,
+                   int64_t ro_stride, int conj, int accumulate, void* stream, const char* name) {
+    const std::string nm(name);
+    if (!in || !out) return tnq_internal_fail(nm + ": bad arguments");
+    Dims d;
+    if (int rc = fill_dims(d, ndim, out_dims, in_strides)) return rc;
+    if (d.size[ndim - 1] != 2) return tnq_internal_fail(nm + ": the last output dimension must be (re, im)");
+    long long total = 1;
+    for (int k = 0; k < ndim; ++k) total *= d.size[k];
+    cplx_fold_kernel<T><<<grid_for(total, 256 * 4), 256, 0, (cudaStream_t)stream>>>(in, out, d, total, ri_stride, ro_stride,
+                                                                                    conj, accumulate);
+    tnq_internal_count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, (nm + " launch").c_str());
+    return 0;
+}
+
+// fold_vec (OUTER = false) / outer_acc (OUTER = true): P, out / T hold (re, im) pairs, 2 * sizeof(T)-byte aligned
+template <typename T, bool OUTER>
+int fold_impl(const T* P, const T* Q, T* out, int64_t A, int64_t D, int64_t C, void* stream, const char* name) {
+    const std::string nm(name);
+    if (!P || !Q || !out || A <= 0 || D <= 0 || C <= 0 || D > 4096) return tnq_internal_fail(nm + ": bad arguments");
+    if (((uintptr_t)P | (uintptr_t)out) & (2 * sizeof(T) - 1))
+        return tnq_internal_fail(nm + (sizeof(T) == 4 ? ": pointers must be 8-byte aligned" : ": pointers must be 16-byte aligned"));
+    const size_t smem = sizeof(T) * 4 * (size_t)D;
+    auto kern = OUTER ? outer_acc_kernel<T> : fold_vec_kernel<T>;
+    if (int rc = allow_smem(kern, smem, "cudaFuncSetAttribute(" + nm + ")")) return rc;
+    kern<<<grid_for(A * C, 256), 256, smem, (cudaStream_t)stream>>>(P, Q, out, A, (int)D, C);
+    tnq_internal_count_launch();
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, (nm + " launch").c_str());
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int tnq_permute_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                    int vec, int conj, void* stream) {
+    return permute_impl(in, out, ndim, out_dims, in_strides, vec, conj, stream, "tnq_permute_f32");
+}
+
+int tnq_permute_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                    int vec, int conj, void* stream) {
+    return permute_impl(in, out, ndim, out_dims, in_strides, vec, conj, stream, "tnq_permute_f64");
+}
+
+int tnq_cplx_expand_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                        int ri_dim, int ro_dim, int conj, void* stream) {
+    return cplx_expand_impl(in, out, ndim, out_dims, in_strides, ri_dim, ro_dim, conj, stream, "tnq_cplx_expand_f32");
+}
+
+int tnq_cplx_expand_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                        int ri_dim, int ro_dim, int conj, void* stream) {
+    return cplx_expand_impl(in, out, ndim, out_dims, in_strides, ri_dim, ro_dim, conj, stream, "tnq_cplx_expand_f64");
 }
 
 int tnq_cplx_fold_f32(const float* in, float* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
                       int64_t ri_stride, int64_t ro_stride, int conj, int accumulate, void* stream) {
-    if (!in || !out) return tnq_internal_fail("tnq_cplx_fold_f32: bad arguments");
-    Dims d;
-    if (int rc = fill_dims(d, ndim, out_dims, in_strides)) return rc;
-    if (d.size[ndim - 1] != 2) return tnq_internal_fail("tnq_cplx_fold_f32: the last output dimension must be (re, im)");
-    long long total = 1;
-    for (int k = 0; k < ndim; ++k) total *= d.size[k];
-    cplx_fold_kernel<<<grid_for(total, 256 * 4), 256, 0, (cudaStream_t)stream>>>(in, out, d, total, ri_stride, ro_stride,
-                                                                                 conj, accumulate);
-    tnq_internal_count_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_cplx_fold_f32 launch");
-    return 0;
+    return cplx_fold_impl(in, out, ndim, out_dims, in_strides, ri_stride, ro_stride, conj, accumulate, stream,
+                          "tnq_cplx_fold_f32");
+}
+
+int tnq_cplx_fold_f64(const double* in, double* out, int ndim, const int64_t* out_dims, const int64_t* in_strides,
+                      int64_t ri_stride, int64_t ro_stride, int conj, int accumulate, void* stream) {
+    return cplx_fold_impl(in, out, ndim, out_dims, in_strides, ri_stride, ro_stride, conj, accumulate, stream,
+                          "tnq_cplx_fold_f64");
 }
 
 int tnq_fold_vec_f32(const float* P, const float* Q, float* out, int64_t A, int64_t D, int64_t C, void* stream) {
-    if (!P || !Q || !out || A <= 0 || D <= 0 || C <= 0 || D > 4096) return tnq_internal_fail("tnq_fold_vec_f32: bad arguments");
-    if (((uintptr_t)P | (uintptr_t)out) & 7) return tnq_internal_fail("tnq_fold_vec_f32: pointers must be 8-byte aligned");
-    const size_t smem = sizeof(float) * 4 * (size_t)D;
-    if (int rc = allow_smem(fold_vec_kernel, smem, "cudaFuncSetAttribute(tnq_fold_vec_f32)")) return rc;
-    fold_vec_kernel<<<grid_for(A * C, 256), 256, smem, (cudaStream_t)stream>>>(P, Q, out, A, (int)D, C);
-    tnq_internal_count_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_fold_vec_f32 launch");
-    return 0;
+    return fold_impl<float, false>(P, Q, out, A, D, C, stream, "tnq_fold_vec_f32");
+}
+
+int tnq_fold_vec_f64(const double* P, const double* Q, double* out, int64_t A, int64_t D, int64_t C, void* stream) {
+    return fold_impl<double, false>(P, Q, out, A, D, C, stream, "tnq_fold_vec_f64");
 }
 
 int tnq_outer_acc_f32(const float* P, const float* Q, float* T, int64_t A, int64_t D, int64_t C, void* stream) {
-    if (!P || !Q || !T || A <= 0 || D <= 0 || C <= 0 || D > 4096) return tnq_internal_fail("tnq_outer_acc_f32: bad arguments");
-    if (((uintptr_t)P | (uintptr_t)T) & 7) return tnq_internal_fail("tnq_outer_acc_f32: pointers must be 8-byte aligned");
-    const size_t smem = sizeof(float) * 4 * (size_t)D;
-    if (int rc = allow_smem(outer_acc_kernel, smem, "cudaFuncSetAttribute(tnq_outer_acc_f32)")) return rc;
-    outer_acc_kernel<<<grid_for(A * C, 256), 256, smem, (cudaStream_t)stream>>>(P, Q, T, A, (int)D, C);
-    tnq_internal_count_launch();
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return tnq_internal_cuda_fail(e, "tnq_outer_acc_f32 launch");
-    return 0;
+    return fold_impl<float, true>(P, Q, T, A, D, C, stream, "tnq_outer_acc_f32");
+}
+
+int tnq_outer_acc_f64(const double* P, const double* Q, double* T, int64_t A, int64_t D, int64_t C, void* stream) {
+    return fold_impl<double, true>(P, Q, T, A, D, C, stream, "tnq_outer_acc_f64");
 }
 
 }  // extern "C"

@@ -27,23 +27,26 @@ for tf in (False, True):
     for _ in range(5): a@b
     e1.record(); torch.cuda.synchronize(); print('cublas 8192^3 tf32' if tf else 'cublas 8192^3 fp32', 2*8192**3*5/e0.elapsed_time(e1)/1e9, 'TFLOP/s')
 del a,b
-# cfg4 probe
+# cfg4 probe: python tools/cfg4_probe.py [chi] [B] [dtype: complex64 | complex128]
 chi = int(sys.argv[1]) if len(sys.argv)>1 else 64
 n, B = 16, int(sys.argv[2]) if len(sys.argv)>2 else 256
-be = tneq_b200.BackendFactory.create_backend('b200', device='cuda:0', dtype='complex64')
+dtype = sys.argv[3] if len(sys.argv)>3 else 'complex64'
+cdt = getattr(torch, dtype)
+print('cfg4 probe:', torch.cuda.get_device_name(dev), 'n', n, 'chi', chi, 'B', B, dtype)
+be = tneq_b200.BackendFactory.create_backend('b200', device='cuda:0', dtype=dtype)
 eng = tneq_b200.EngineSiamese(backend=be, strategy_mode='balanced', mx_K=chi)
 g = tneq_b200.QCTNHelper.generate_example_graph(n=n, graph_type='mps', dim_char=str(chi))
 torch.manual_seed(0)
 t=time.time(); q = tneq_b200.QCTN(g, backend=be); torch.cuda.synchronize(); print('qctn init', time.time()-t)
 for c in q.cores: q.cores_weights[c].requires_grad_(True)
-st = [torch.zeros(chi, device=dev, dtype=torch.complex64) for _ in range(n)]
+st = [torch.zeros(chi, device=dev, dtype=cdt) for _ in range(n)]
 for s in st: s[-1]=1
-eye = torch.eye(chi, dtype=torch.complex64, device=dev).expand(B,chi,chi)
+eye = torch.eye(chi, dtype=cdt, device=dev).expand(B,chi,chi)
 out = eng.contract_with_compiled_strategy(q, st, [eye]*n); torch.cuda.synchronize()
 print('KAT-1 identity measurement -> ', out[:4], 'max dev from 1:', (out-1).abs().max().item())
 x = torch.randn(B,n, device=dev)*0.3
 mx,_ = eng.generate_data(x, K=chi, ret_type='TNTensor')
-for it in range(3):
+for it in range(4):
     torch.cuda.synchronize(); t=time.time()
     l0 = _lib.launch_count()
     loss, grads = eng.contract_with_compiled_strategy_for_gradient(q, st, mx)
