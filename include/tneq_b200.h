@@ -264,6 +264,28 @@ int tnq_sgdg_step(float* const* params, const float* const* grads, float* const*
  * traffic and no host synchronisation. */
 int tnq_sgdg_step_flat(float* params, const float* grads, float* velocity, const int64_t* offsets, const int* rows,
                        const int* cols, int ncores, int max_cols, float lr, float momentum, void* stream);
+/* The same two steps for complex64 (_c64), float64 (_f64) and complex128 (_c128) cores.  Complex matrices are
+ * interleaved (re, im) pairs; offsets, rows and cols count complex elements.  Transposes become conjugate
+ * transposes (V = momentum * V - g^H, W = W^ - W^H, p_new = Y^H), as in the reference's complex branch.
+ * rows[i] <= cols[i] <= TNQ_SGDG_MAX_COLS_<dtype>: the matrices of one core share an sm_100 block's shared
+ * memory, six of cols x (cols + 1) elements. */
+#define TNQ_SGDG_MAX_COLS_C64 64
+#define TNQ_SGDG_MAX_COLS_F64 64
+#define TNQ_SGDG_MAX_COLS_C128 48
+int tnq_sgdg_step_c64(float* const* params, const float* const* grads, float* const* velocity, const int* rows,
+                      const int* cols, int ncores, int max_cols, float lr, float momentum, void* stream);
+int tnq_sgdg_step_flat_c64(float* params, const float* grads, float* velocity, const int64_t* offsets, const int* rows,
+                           const int* cols, int ncores, int max_cols, float lr, float momentum, void* stream);
+int tnq_sgdg_step_f64(double* const* params, const double* const* grads, double* const* velocity, const int* rows,
+                      const int* cols, int ncores, int max_cols, double lr, double momentum, void* stream);
+int tnq_sgdg_step_flat_f64(double* params, const double* grads, double* velocity, const int64_t* offsets,
+                           const int* rows, const int* cols, int ncores, int max_cols, double lr, double momentum,
+                           void* stream);
+int tnq_sgdg_step_c128(double* const* params, const double* const* grads, double* const* velocity, const int* rows,
+                       const int* cols, int ncores, int max_cols, double lr, double momentum, void* stream);
+int tnq_sgdg_step_flat_c128(double* params, const double* grads, double* velocity, const int64_t* offsets,
+                            const int* rows, const int* cols, int ncores, int max_cols, double lr, double momentum,
+                            void* stream);
 
 /*
  * One-shot all-reduce of the packed gradient + loss buffer of one training step over NVLink peer

@@ -16,7 +16,9 @@ EXPORTS = ["tnq_device_check", "tnq_plan_create", "tnq_plan_destroy", "tnq_plan_
            "tnq_plan_num_outputs", "tnq_plan_query", "tnq_plan_run", "tnq_gemm_tf32x3", "tnq_gemm_tf32x3_view", "tnq_gemm_tf32x3_bk", "tnq_gemm_kernel_attrs", "tnq_permute_f32", "tnq_fold_vec_f32", "tnq_outer_acc_f32", "tnq_cplx_expand_f32",
            "tnq_cplx_fold_f32", "tnq_gemm_f64", "tnq_permute_f64", "tnq_fold_vec_f64", "tnq_outer_acc_f64", "tnq_cplx_expand_f64",
            "tnq_cplx_fold_f64", "tnq_mps_chain", "tnq_mps_chain_workspace_bytes", "tnq_mps_chain_x", "tnq_mps_chain_sample", "tnq_mps_ladder",
-           "tnq_mps_ladder_workspace_bytes", "tnq_mps_ladder2", "tnq_mps_ladder2_workspace_bytes", "tnq_mps_ladder2_geometry", "tnq_allreduce_oneshot", "tnq_allreduce_oneshot_words", "tnq_allreduce_set_timeout_ms", "tnq_sgdg_step", "tnq_sgdg_step_flat", "tnq_launch_count",
+           "tnq_mps_ladder_workspace_bytes", "tnq_mps_ladder2", "tnq_mps_ladder2_workspace_bytes", "tnq_mps_ladder2_geometry", "tnq_allreduce_oneshot", "tnq_allreduce_oneshot_words", "tnq_allreduce_set_timeout_ms", "tnq_sgdg_step", "tnq_sgdg_step_flat",
+           "tnq_sgdg_step_c64", "tnq_sgdg_step_flat_c64", "tnq_sgdg_step_f64", "tnq_sgdg_step_flat_f64", "tnq_sgdg_step_c128",
+           "tnq_sgdg_step_flat_c128", "tnq_launch_count",
            "tnq_last_error"]
 
 
@@ -93,6 +95,10 @@ def load():
                                        c_float, c_void_p]
     lib.tnq_sgdg_step.argtypes = [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_float, c_float,
                                   c_void_p]
+    # complex64 / float64 / complex128 siblings: the same arguments, lr and momentum in double for the double types
+    for sfx, real in (("c64", c_float), ("f64", c_double), ("c128", c_double)):
+        getattr(lib, f"tnq_sgdg_step_{sfx}").argtypes = lib.tnq_sgdg_step.argtypes[:7] + [real, real, c_void_p]
+        getattr(lib, f"tnq_sgdg_step_flat_{sfx}").argtypes = lib.tnq_sgdg_step_flat.argtypes[:8] + [real, real, c_void_p]
     _lib = lib
     return lib
 

@@ -446,7 +446,8 @@ class _Call:
             grads, res = self._gemm_backward(cores, seed_fn)
             return box["loss"], grads, self._shape_result(res.reshape(self.nsamples, -1))
         prog = self.bound.program("train")
-        outs = prog.run(self.nsamples, self._inputs(prog, cores), scalars=(log_scale, 1.0 / self.nsamples))
+        outs = prog.run(self.nsamples, self._inputs(prog, cores), scalars=(log_scale, 1.0 / self.nsamples),
+                        one_buffer=True)
         loss = outs[prog.prog.output_index(("loss", 0))][0]
         values = self._shape_result(outs[prog.prog.output_index(("result", 0))])
         return loss, self._grads(prog, outs, cores), values

@@ -7,6 +7,7 @@ CUDA stream go down; nothing but an error code comes back.
 from __future__ import annotations
 
 import ctypes
+import math
 from ctypes import byref, c_double, c_int64, c_void_p
 from typing import Dict, List, Sequence, Tuple
 
@@ -55,10 +56,13 @@ class DeviceProgram:
             self._info[nsamples] = ri
         return self._info[nsamples]
 
-    def run(self, nsamples: int, inputs: Sequence[Tuple[torch.Tensor, int, int]], scalars=(0.0, 1.0)):
+    def run(self, nsamples: int, inputs: Sequence[Tuple[torch.Tensor, int, int]], scalars=(0.0, 1.0),
+            one_buffer: bool = False):
         """inputs[i] = (tensor whose data_ptr is the slot's base, stride_hi, stride_lo) in
         program order; strides in real elements.  Returns the list of output tensors
-        (batched: [nsamples, elems]; shared: [elems]) of the program's real dtype."""
+        (batched: [nsamples, elems]; shared: [elems]) of the program's real dtype; with one_buffer they are
+        views of ONE allocation, every slot starting on a 256-byte boundary (the optimizer's table-free SGDG
+        launch takes gradients that way, optim/steps.py)."""
         ri = self.info(nsamples)
         if self._ws is None or self._ws.numel() < ri.workspace_bytes:
             self._ws = torch.empty(int(ri.workspace_bytes), dtype=torch.uint8, device=self.device)
@@ -70,8 +74,18 @@ class DeviceProgram:
             self._in_ptrs[i] = t.data_ptr()
             self._hi[i], self._lo[i] = int(hi), int(lo)
         outs = []
-        for j, s in enumerate(self.prog.outputs):
-            o = torch.empty((nsamples, s.elems) if s.batched else (s.elems,), dtype=self.real_dtype, device=self.device)
+        shapes = [(nsamples, s.elems) if s.batched else (s.elems,) for s in self.prog.outputs]
+        if one_buffer:
+            align = 256 * 8 // torch.finfo(self.real_dtype).bits        # elements per 256 bytes
+            starts = [0]
+            for shp in shapes:
+                starts.append(starts[-1] + -(-math.prod(shp) // align) * align)
+            buf = torch.empty(starts[-1], dtype=self.real_dtype, device=self.device)
+        for j, shp in enumerate(shapes):
+            if one_buffer:
+                o = buf[starts[j]: starts[j] + math.prod(shp)].view(shp)
+            else:
+                o = torch.empty(shp, dtype=self.real_dtype, device=self.device)
             outs.append(o)
             self._out_ptrs[j] = o.data_ptr()
         self._scalars[0], self._scalars[1] = float(scalars[0]), float(scalars[1])

@@ -8,9 +8,10 @@ Stiefel-manifold SGD with a Cayley retraction used by the examples
 the update acts on tensor*scale with grad/scale and re-wraps (:205-266).
 
 These are small dense per-core operations (K^2 x K^2 matrices).  'sgdg', the
-method the examples use, runs for all float32 cores of a network as ONE launch
-of csrc/tnq_sgdg.cu (one CTA per core); the other methods, complex cores and
-cores wider than TNQ_SGDG_MAX_COLS go through torch on the device.
+method the examples use, runs for all float32, complex64, float64 and complex128
+cores of a network as ONE launch of csrc/tnq_sgdg.cu (one CTA per core); the
+other methods and cores wider than their dtype's TNQ_SGDG_MAX_COLS* go through
+torch on the device.
 """
 from __future__ import annotations
 
@@ -109,6 +110,13 @@ def _rmsprop(params, grads, state, hp):
 
 
 SGDG_MAX_COLS = 64          # TNQ_SGDG_MAX_COLS, include/tneq_b200.h
+# per dtype: suffix of the tnq_sgdg_step entry points and the widest matrix they take (TNQ_SGDG_MAX_COLS*)
+SGDG_KERNELS = {torch.float32: ("", SGDG_MAX_COLS), torch.complex64: ("_c64", 64), torch.float64: ("_f64", 64),
+                torch.complex128: ("_c128", 48)}
+# The kernel divides every row by its norm + 1e-8; the reference takes a retracted core's rows as they are.  Stored
+# 2^27 times larger, a unit row comes out of that division as itself to within rounding in float64 as well
+# (1e-8 / 2^27 < 1e-16).  float32 keeps the unscaled retraction: 1e-8 is below its rounding at 1.
+_RETRACT_SCALE = {torch.float32: 1.0}
 
 
 @functools.lru_cache(maxsize=4096)
@@ -121,6 +129,16 @@ def _matrix_shape(shp):
     return (int(shp[0]), int(shp[1])) if len(shp) == 2 else (0, 0)
 
 
+def sgdg_kernel_eligible(dtype, shape, device_type) -> bool:
+    """Whether the Cayley step of a core of this dtype and shape runs in csrc/tnq_sgdg.cu: a Stiefel core
+    (rows <= cols as the step's matrix) on a CUDA device, no wider than the maximum of its dtype."""
+    kernel = SGDG_KERNELS.get(dtype)
+    if kernel is None or device_type != "cuda":
+        return False
+    r, c = _matrix_shape(tuple(shape))
+    return 1 <= r <= c <= kernel[1]
+
+
 def _qr_retract(unity):
     qm, rm = torch.linalg.qr(unity.T, mode="reduced")
     d = torch.diag(rm)
@@ -131,23 +149,27 @@ def _sgdg_flat_step(params, grads, state, lr, mom, out):
     """All cores in one launch with NO per-step host-to-device traffic: parameters are packed into one
     fresh buffer (the reference returns new tensors), gradients already sit in one buffer (the fused
     contraction routes return them as views of it), the momentum buffers live in one persistent
-    buffer, and the offset table is static per network (tnq_sgdg_step_flat).  Returns False when the
-    gradients are not views of one float32 buffer."""
+    buffer, and the offset table is static per network (tnq_sgdg_step_flat*).  All cores have one dtype; complex
+    gradients may be complex views of one real buffer (view_as_complex), offsets count elements of the cores'
+    dtype.  Returns False when the gradients are not views of one buffer."""
     from .. import _lib
+    dtype = params[0].dtype
+    esize = params[0].element_size()
     base = getattr(grads[0], "_base", None)
-    if base is None or not base.is_cuda or base.dtype != torch.float32 or not base.is_contiguous():
+    if (base is None or not base.is_cuda or base.dtype not in (dtype, dtype.to_real()) or not base.is_contiguous()
+            or base.data_ptr() % esize):
         return False
     b0 = base.data_ptr()
     g_off = []
     for g in grads:
-        if getattr(g, "_base", None) is not base or not g.is_contiguous():
+        if getattr(g, "_base", None) is not base or not g.is_contiguous() or (g.data_ptr() - b0) % esize:
             return False
-        g_off.append((g.data_ptr() - b0) // 4)
+        g_off.append((g.data_ptr() - b0) // esize)
     lib = _lib.load()
     dev = params[0].device
     shapes = [_matrix_shape(p.shape) for p in params]
     sizes = [r * c for r, c in shapes]
-    key = (tuple(shapes), tuple(g_off))
+    key = (dtype, tuple(shapes), tuple(g_off))
     with torch.cuda.device(dev):
         if state.get("_flat_key") != key:          # first step (or a different network): build the static tables
             p_off = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
@@ -155,7 +177,7 @@ def _sgdg_flat_step(params, grads, state, lr, mom, out):
             state["_flat_key"] = key
             state["_flat_offs"] = torch.from_numpy(table).to(dev)
             state["_flat_dims"] = torch.tensor([[r for r, _ in shapes], [c for _, c in shapes]], dtype=torch.int32, device=dev)
-            vflat = torch.zeros(int(sum(sizes)), dtype=torch.float32, device=dev)
+            vflat = torch.zeros(int(sum(sizes)), dtype=dtype, device=dev)
             for i, (off, n) in enumerate(zip(p_off, sizes)):
                 old = state["momentum_buffer"][i]
                 r, c = shapes[i]
@@ -168,7 +190,7 @@ def _sgdg_flat_step(params, grads, state, lr, mom, out):
             # two persistent parameter buffers used alternately: the cores of step i+2 live where those of step i
             # lived, so a training loop presents only two sets of addresses (CUDA-graph replay, DataParallelTrainer.
             # enable_cuda_graphs); the tensors returned two steps ago are overwritten
-            bufs = state.setdefault("_flat_p", [torch.empty(int(sum(sizes)), dtype=torch.float32, device=dev) for _ in range(2)])
+            bufs = state.setdefault("_flat_p", [torch.empty(int(sum(sizes)), dtype=dtype, device=dev) for _ in range(2)])
             flat = bufs[state.get("_flat_turn", 0) & 1]
             state["_flat_turn"] = state.get("_flat_turn", 0) + 1
             torch.cat([p.reshape(-1) for p in params], out=flat)
@@ -181,21 +203,22 @@ def _sgdg_flat_step(params, grads, state, lr, mom, out):
             if rng.randint(1, 101) == 1:
                 r, c = shapes[n]
                 x = flat[p_off[n]: p_off[n] + sizes[n]].view(r, c)
-                x.copy_(_qr_retract(x / (torch.norm(x, p=2, dim=1, keepdim=True) + 1e-8)))
+                x.copy_(_RETRACT_SCALE.get(dtype, 2.0 ** 27) * _qr_retract(x / (torch.norm(x, p=2, dim=1, keepdim=True) + 1e-8)))
         dims, offs = state["_flat_dims"], state["_flat_offs"]
-        _lib.check(lib.tnq_sgdg_step_flat(flat.data_ptr(), b0, state["_flat_v"].data_ptr(), offs.data_ptr(),
-                                          dims[0].data_ptr(), dims[1].data_ptr(), len(params), max(c for _, c in shapes),
-                                          float(lr), float(mom), torch.cuda.current_stream().cuda_stream))
+        step = getattr(lib, "tnq_sgdg_step_flat" + SGDG_KERNELS[dtype][0])
+        _lib.check(step(flat.data_ptr(), b0, state["_flat_v"].data_ptr(), offs.data_ptr(), dims[0].data_ptr(),
+                        dims[1].data_ptr(), len(params), max(c for _, c in shapes), float(lr), float(mom),
+                        torch.cuda.current_stream().cuda_stream))
     for n, p in enumerate(params):
         out[n] = flat[p_off[n]: p_off[n] + sizes[n]].view(p.shape)
     return True
 
 
 def _sgdg_kernel_step(idx, params, grads, state, lr, mom, out):
-    """All eligible cores in one launch of tnq_sgdg_step (csrc/tnq_sgdg.cu)."""
+    """All eligible cores, of one dtype, in one launch of tnq_sgdg_step* (csrc/tnq_sgdg.cu)."""
     from .. import _lib
     lib = _lib.load()
-    dev = params[idx[0]].device
+    dev, dtype = params[idx[0]].device, params[idx[0]].dtype
     shapes = [_matrix_shape(params[i].shape) for i in idx]
     sizes = [r * c for r, c in shapes]
     with torch.cuda.device(dev):
@@ -209,14 +232,14 @@ def _sgdg_kernel_step(idx, params, grads, state, lr, mom, out):
                 r, c = shapes[n]
                 off = sum(sizes[:n])
                 x = flat[off: off + sizes[n]].view(r, c)
-                x.copy_(_qr_retract(x / (torch.norm(x, p=2, dim=1, keepdim=True) + 1e-8)))
+                x.copy_(_RETRACT_SCALE.get(dtype, 2.0 ** 27) * _qr_retract(x / (torch.norm(x, p=2, dim=1, keepdim=True) + 1e-8)))
             if state["momentum_buffer"][i] is None:
                 r, c = shapes[n]
-                state["momentum_buffer"][i] = torch.zeros(c, r, dtype=torch.float32, device=dev)
+                state["momentum_buffer"][i] = torch.zeros(c, r, dtype=dtype, device=dev)
             elif not state["momentum_buffer"][i].is_contiguous():
                 state["momentum_buffer"][i] = state["momentum_buffer"][i].contiguous()
         vs = [state["momentum_buffer"][i] for i in idx]
-        offs = np.concatenate([[0], np.cumsum(sizes)[:-1]]) * 4
+        offs = np.concatenate([[0], np.cumsum(sizes)[:-1]]) * flat.element_size()
         table = np.empty((3, len(idx)), dtype=np.int64)
         table[0] = flat.data_ptr() + offs
         table[1] = [g.data_ptr() for g in gs]
@@ -228,9 +251,9 @@ def _sgdg_kernel_step(idx, params, grads, state, lr, mom, out):
                                                device=dev)
         dims = state["_sgdg_dims"]
         tdev = torch.from_numpy(table).to(dev)
-        _lib.check(lib.tnq_sgdg_step(tdev[0].data_ptr(), tdev[1].data_ptr(), tdev[2].data_ptr(), dims[0].data_ptr(),
-                                     dims[1].data_ptr(), len(idx), max(c for _, c in shapes), float(lr), float(mom),
-                                     torch.cuda.current_stream().cuda_stream))
+        step = getattr(lib, "tnq_sgdg_step" + SGDG_KERNELS[dtype][0])
+        _lib.check(step(tdev[0].data_ptr(), tdev[1].data_ptr(), tdev[2].data_ptr(), dims[0].data_ptr(), dims[1].data_ptr(),
+                        len(idx), max(c for _, c in shapes), float(lr), float(mom), torch.cuda.current_stream().cuda_stream))
     off = 0
     for n, i in enumerate(idx):
         out[i] = flat[off: off + sizes[n]].view(params[i].shape)
@@ -244,16 +267,16 @@ def _sgdg(params, grads, state, hp):
     if "momentum_buffer" not in state:
         state["momentum_buffer"] = [None] * len(params)
     out = [None] * len(params)
-    fast = []
+    fast = {}                   # dtype -> indices of the cores the kernel of that dtype takes
     if stiefel and hp.get("device_kernel", True):
         for i, (p, g) in enumerate(zip(params, grads)):
-            r, c = _matrix_shape(p.shape)
-            if (p.is_cuda and p.dtype == torch.float32 and g.dtype == torch.float32 and 1 <= r <= c <= SGDG_MAX_COLS):
-                fast.append(i)
-    if fast and len(fast) == len(params) and _sgdg_flat_step(params, grads, state, lr, mom, out):
+            if g.dtype == p.dtype and sgdg_kernel_eligible(p.dtype, p.shape, p.device.type):
+                fast.setdefault(p.dtype, []).append(i)
+    if (len(fast) == 1 and len(next(iter(fast.values()))) == len(params)
+            and _sgdg_flat_step(params, grads, state, lr, mom, out)):
         return out, state
-    if fast:
-        _sgdg_kernel_step(fast, params, grads, state, lr, mom, out)
+    for idx in fast.values():
+        _sgdg_kernel_step(idx, params, grads, state, lr, mom, out)
     for i, (p, g) in enumerate(zip(params, grads)):
         if out[i] is not None:
             continue
