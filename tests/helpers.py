@@ -127,6 +127,58 @@ def mps_f64_value(amp):
     return amp.real ** 2 + amp.imag ** 2 if amp.is_complex() else amp
 
 
+def ladder_layers(graph, K):
+    """(layer1, layer2): the core names of the two layers of a merged MPS network, as the ladder route reads them
+    off the plan (plan.mps_ladder(), used by b200_strategy._ladder)."""
+    import tneq_b200
+    from tneq_b200.contractor.plan import ContractionPlan
+    q = tneq_b200.QCTN(graph)
+    n = q.nqubits
+    plan = ContractionPlan(q.adjacency_table, n, {c: (K,) * 4 for c in q.cores}, {i: K for i in range(n)},
+                           {i: ("a", K, K) for i in range(n)}, "float32")
+    lad = plan.mps_ladder()
+    assert lad is not None and lad[0] == K
+    return lad[1], lad[2]
+
+
+def ladder_f64(cores_a, cores_x, states, mxs):
+    """The two-layer merged MPS sweep (QCTN.merge(mps_n, mps_n); greedy groups
+    'cdef,eghi,c,ahj,klmn,mojp,k,d,l->agnpfio', 'cdef,ghij,aik,lmno,pqkr,aelpcgn,d,m->ahorfjq',
+    'cdef,gfhi,ahj,klmn,onjp,aekocgm,d,l->api', 'acd,adc->a') restated pairwise in the order of DESIGN 3d, on whatever
+    device and dtype the inputs have: the float64 yardstick of the ladder kernels, where the oracle's left-to-right
+    einsum of a middle group builds B K^12 intermediates.  cores_a / cores_x: the n-1 cores of the first / second
+    layer (plan.mps_ladder() order), A_q and X_q acting on wires (q, q+1).  Per qubit and sample the largest
+    intermediate has K^7 entries.  Real networks only (what the ladder kernels take).  Returns the values (B,).
+    Pinned to the oracle by tests/test_large_bond_yardstick.py."""
+    n = len(states)
+    a0, x0 = cores_a[0], cores_x[0]
+    # first group: env[a,g,n,p,f,i,o] (ket: A_0 out on wire 1 = f, X_0 in / out on wire 1 = g / i; bra: n, o, p)
+    v = torch.einsum("cdef,c,d->ef", a0, states[0], states[1])
+    t = torch.einsum("ef,eghi->fghi", v, x0)
+    u = torch.einsum("ahj,mojp->ahmop", mxs[0], x0)
+    u = torch.einsum("mn,ahmop->ahnop", v, u)
+    env = torch.einsum("fghi,ahnop->agnpfio", t, u)
+    for q in range(1, n - 2):
+        a, x = cores_a[q], cores_x[q]
+        bs = torch.einsum("cdef,d->cef", a, states[q + 1])
+        # A: T2[f,o,g,p] = sum_{c,e,l,n} Bs[c,e,f] Bs[l,n,o] E[c,l,n,p,e,g]
+        t1 = torch.einsum("aelpcgn,cef->alnpgf", env, bs)
+        t2 = torch.einsum("alnpgf,lno->afogp", t1, bs)
+        # B: U[i,p,q,r] = sum_k M[i,k] X[p,q,k,r]
+        u = torch.einsum("aik,pqkr->aipqr", mxs[q], x)
+        # C: E'[f,o,q,r,h,j] = sum_{g,i,p} T2[f,o,g,p] U[i,p,q,r] X[g,h,i,j]
+        w = torch.einsum("afogp,aipqr->afogiqr", t2, u)
+        env = torch.einsum("afogiqr,ghij->ahorfjq", w, x)
+    a, x = cores_a[n - 2], cores_x[n - 2]
+    bs = torch.einsum("cdef,d->cef", a, states[n - 1])
+    t1 = torch.einsum("aekocgm,cef->akogmf", env, bs)
+    t2 = torch.einsum("akogmf,kmn->aogfn", t1, bs)
+    u = torch.einsum("ahj,onjp->ahonp", mxs[n - 2], x)
+    w = torch.einsum("aogfn,ahonp->agfhp", t2, u)
+    out = torch.einsum("agfhp,gfhi->api", w, x)
+    return torch.einsum("acd,adc->a", out, mxs[n - 1])
+
+
 # ---- which GEMM variant a large-bond launch takes --------------------------------------------------------------------
 GEMM_TILE = 128          # BM = BN of csrc/tnq_gemm.cu
 GEMM_BK = 32             # BK of csrc/tnq_gemm.cu
@@ -219,3 +271,42 @@ LARGE_BOND_CASES = [
     ("complex64", 128, 3, 2, {("view", True)} | _FOLD,
      {("view", True)} | _FOLD),
 ]
+
+
+# ---- which register-resident kernels a call launches ----------------------------------------------------------------
+class KernelRecorder:
+    """Names of this library's CUDA kernels launched inside the `with` block, recorded with torch.profiler (CUDA
+    activity).  The profiler reports demangled template instances, e.g.
+    'void (anonymous namespace)::tnq_chain_kernel<3, 1>(...)'; `names` keeps the instance ('tnq_chain_kernel<3, 1>').
+    A block that launches no tnq_ kernel at all fails: a profiler that cannot see kernel names must not turn a
+    coverage assertion into no assertion."""
+
+    def __enter__(self):
+        from torch.profiler import ProfilerActivity, profile
+        torch.cuda.synchronize()
+        self._prof = profile(activities=[ProfilerActivity.CUDA])
+        self._prof.__enter__()
+        return self
+
+    def __exit__(self, *exc):
+        import re
+        torch.cuda.synchronize()
+        self._prof.__exit__(*exc)
+        if exc[0] is not None:
+            return False
+        found = set()
+        for ev in self._prof.events():
+            m = re.search(r"tnq_\w+(<[^<>()]*>)?", ev.name)
+            if m:
+                found.add(m.group(0))
+        assert found, "the profiler saw no tnq_ kernel"
+        self.names = found
+        return False
+
+    def check(self, expected):
+        """Every expected name (a template instance, or a prefix for non-template kernels) was launched, and nothing
+        else of this library was."""
+        for e in expected:
+            assert any(n.startswith(e) for n in self.names), (e, sorted(self.names))
+        for n in self.names:
+            assert any(n.startswith(e) for e in expected), (n, sorted(expected))

@@ -223,10 +223,12 @@ def test_sampling_prefix_environments_equal_contraction_methods(built_lib):
         assert tuple(out["prefix"].shape) == (S, nq)
         assert launches["prefix"] == 1 and launches["auto"] == 1 and launches["grid"] >= nq
         assert (out["prefix"] >= -5).all() and (out["prefix"] <= 5).all()
-        # the inverse CDF is continuous in the densities: float32 round-off in the running sums moves a sample by
-        # ~1e-6 of the grid spacing, a flipped `cdf < u` comparison leaves the interpolated value continuous
-        # (the bulk agrees to ~1e-6; where a grid cell carries almost no probability the reference's own formula
-        # (u - c0) / (c1 - c0 + 1e-10) divides two round-off-sized numbers, hence a bound in units of the cell)
+        # float32 round-off in the running sums moves a sample by ~1e-6 of the grid spacing (the bulk agrees to
+        # ~1e-6; where a grid cell carries almost no probability the reference's own formula (u - c0) / (c1 - c0 + 1e-10)
+        # divides two round-off-sized numbers, hence a bound in units of the cell).  A flipped `cdf < u` comparison is
+        # NOT continuous: the formula extrapolates from the first CDF value not below u, so a flip moves y by
+        # dx (1 - d[idx+1] / d[idx+2]).  It needs u within the running sums' round-off of a CDF value, which these few
+        # draws do not meet; tests/test_gpu_register_kernels.py checks such flips at 227 559 draws.
         cell = 10.0 / (G - 1)
         for other in ("grid", "linear"):
             diff = (out["prefix"] - out[other]).abs()
